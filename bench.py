@@ -21,6 +21,9 @@ across ranks, no data-path collective): weak scaling.
           C4 as a 120-frame video through the mocap skeleton path, wall clock).
   tiles : (N > 1) ONE frame of C2 / C3 / C5 cut across the N GPUs of the box (strong scaling of the
           single-frame path), driven by rank 0 after the frame-sharded legs.
+  --dump-outputs DIR : DIR/frame_r<rank>.npy, the frame each rank's e2e leg received in its last timed step (float32
+          copy of the u8 frame; a fixed seeded pixel sample where N full frames would pass 64 MB).  Frames and seeds depend
+          only on --gpus / --warmup / --steps, so two builds run with the same arguments can be compared pixel for pixel.
   --impl reference : the reference's own CPU renderer (oracle/_ref, the unmodified
           reference sources compiled here) on all host cores, one process per core on
           a fixed stratified sample of the same frame.
@@ -450,6 +453,10 @@ def run_ours(args):
         dev.render(settings, tile, out=host_frame)       # kernels + D2H of the u8 frame
     barrier()
     e2e_ms = 1e3 * (time.perf_counter() - t0)
+    if args.dump_outputs:
+        # the device-resident leg's last step rendered the same frame and seed into device memory only
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, f"frame_r{rank}.npy"), dump_sample(host_frame, world))
 
     def maxr(x):
         return shard.max_over_ranks(x, dist if world > 1 else None, device="cuda")
@@ -577,6 +584,20 @@ def roofline_blocks(dev, settings, tile, step_s, clock_info, local, launches, st
     return out
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_sample(frame, world):
+    """The frame as float32 (h, w, 3); when the frames of all ranks would exceed DUMP_BYTES, the same seeded sample of
+    pixels on every rank instead, as float32 (n, 3) in ascending row-major pixel order."""
+    f = frame.astype(np.float32)
+    budget = (DUMP_BYTES - 4096 * world) // world
+    if f.nbytes <= budget:
+        return f
+    keep = np.sort(np.random.default_rng(0).choice(f.shape[0] * f.shape[1], budget // (3 * 4), replace=False))
+    return f.reshape(-1, 3)[keep]
+
+
 def h2d_scene_bytes(dev, scene):
     """Bytes drt_scene_update_prims uploads per call (both precisions' geom/prim/node/light tables
     are small; counted from the POD input the host hands over)."""
@@ -593,7 +614,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="only the timed legs (A/B runs, ncu launch lists)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write each rank's frame of the last timed step as DIR/frame_r<rank>.npy (float32, PPM row order)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference leg times a sample of the frame and keeps no image")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -1,11 +1,15 @@
-"""Randomised pin of the CPU restatement on the compiled reference (build container only: needs oracle/_ref and the
-reference's assets).  Beyond the 15 stored fixtures: reference scene builders at random frames with random settings
-(resolution, spp, aperture, lobes, depth, switches, seed), rendered by the UNMODIFIED reference rayColor and by
-oracle/drt_oracle.cpp under the same sequential sample stream -- floats and abort masks must agree to the bit."""
+"""Randomised pin of the CPU restatement on the compiled reference.  Beyond the 15 stored fixtures: reference scene builders
+at random frames with random settings (resolution, spp, aperture, lobes, depth, switches, seed), and generated scenes
+loaded into the reference, rendered by the UNMODIFIED reference rayColor and by oracle/drt_oracle.cpp under the same
+sequential sample stream -- floats and abort masks must agree to the bit.  The comparisons against the live reference
+need oracle/_ref and the reference's tree; for the generated scenes the reference's images are also stored, as digests
+(tests/golden/reference_pins.json), so those cases are checked without the reference too."""
 import os
 
 import numpy as np
 import pytest
+
+from conftest import assert_pinned
 
 BUILDERS = ["hw4", "reflectance", "dof", "spherelight", "spheres", "checkertexture", "texture", "textureog", "window",
             "staircase", "rectprism", "checkercylinder", "chkpt2", "boundary"]
@@ -14,6 +18,31 @@ BUILDERS = ["hw4", "reflectance", "dof", "spherelight", "spheres", "checkertextu
 def _have_reference():
     from oracle.harness import ref_available, REFERENCE_ROOT
     return ref_available() and os.path.isdir(os.path.join(REFERENCE_ROOT, "textures"))
+
+
+def _reference_render(scene, s, mocap):
+    from oracle.harness import Ref
+    r = Ref(mocap=mocap)
+    r.reset()
+    r.load(scene)
+    r.set_settings(s)
+    r.rng(1, s.seed, 0)
+    ref_img, ref_ab, _ = r.render_loop(int(s.frame), reset_policy=1, seed=s.seed)
+    return ref_img, ref_ab
+
+
+def _pinned_render(key, scene, s, mocap=False):
+    """The restatement's image of `scene` is the reference's: compared with the compiled reference where it is built,
+    and with the stored pin everywhere."""
+    from oracle.harness import Oracle, ORACLE_STREAM
+    img, ab, cnt, _ = Oracle(scene).render(s, mode=ORACLE_STREAM)
+    live = _have_reference()
+    if live:
+        ref_img, ref_ab = _reference_render(scene, s, mocap)
+        assert (ab == ref_ab).all(), (key, "abort masks differ")
+        assert np.array_equal(ref_img, img, equal_nan=True), (key, float(np.nanmax(np.abs(ref_img - img))))
+    assert_pinned(key, img, ab, matched_reference=live)
+    return img, ab, cnt
 
 
 @pytest.mark.parametrize("seed", range(28))
@@ -104,20 +133,9 @@ def test_restatement_matches_reference_on_random_scenes(oracle_lib, seed):
     """Scenes no builder of the reference produces (fuzz_cases.random_scene: random spheres, cylinders, triangles,
     rectangles with their corners in ANY order -- a third of them therefore with D - A a diagonal, Q20 -- checkerboards,
     all three light kinds) loaded INTO the compiled reference: the restatement reproduces them to the bit."""
-    if not _have_reference():
-        pytest.skip("reference tree not present (GPU box): pinned by the stored fixtures instead")
     from fuzz_cases import random_scene
-    from oracle.harness import Ref, Oracle, ORACLE_STREAM
     _, scene, s = random_scene(seed)
-    r = Ref(mocap=False)
-    r.reset()
-    r.load(scene)
-    r.set_settings(s)
-    r.rng(1, s.seed, 0)
-    ref_img, ref_ab, _ = r.render_loop(int(s.frame), reset_policy=1, seed=s.seed)
-    img, ab, _, _ = Oracle(scene).render(s, mode=ORACLE_STREAM)
-    assert (ab == ref_ab).all(), (seed, "abort masks differ")
-    assert np.array_equal(ref_img, img, equal_nan=True), (seed, float(np.nanmax(np.abs(ref_img - img))))
+    _pinned_render(f"random_scenes/{seed}", scene, s)
 
 
 @pytest.mark.parametrize("seed", range(30))
@@ -125,60 +143,27 @@ def test_restatement_matches_reference_on_random_scenes_with_its_own_blur(oracle
     """fuzz_cases.random_refblur_scene: the random scenes in the REFERENCE's blur mode after frame_prism -- every rectangle
     and checkerboard moves in y during the blur re-traces (the reference names them all "rectangle"), leaf boxes are bumped,
     interior ones are not -- loaded into the compiled reference: reproduced to the bit."""
-    if not _have_reference():
-        pytest.skip("reference tree not present (GPU box): pinned by the stored fixtures instead")
     from fuzz_cases import random_refblur_scene
-    from oracle.harness import Ref, Oracle, ORACLE_STREAM
     _, scene, s = random_refblur_scene(seed)
-    r = Ref(mocap=False)
-    r.reset()
-    r.load(scene)
-    r.set_settings(s)
-    r.rng(1, s.seed, 0)
-    ref_img, ref_ab, _ = r.render_loop(int(s.frame), reset_policy=1, seed=s.seed)
-    img, ab, _, _ = Oracle(scene).render(s, mode=ORACLE_STREAM)
-    assert (ab == ref_ab).all(), (seed, "abort masks differ")
-    assert np.array_equal(ref_img, img, equal_nan=True), (seed, float(np.nanmax(np.abs(ref_img - img))))
+    _pinned_render(f"random_refblur_scenes/{seed}", scene, s)
 
 
 @pytest.mark.parametrize("seed", range(8))
 def test_restatement_matches_reference_on_big_random_scenes(oracle_lib, seed):
     """fuzz_cases.random_big_scene: 257 .. 700 small shapes over a floor (the scenes on which the CUDA path gathers through
     its tree over the geoms) loaded INTO the compiled reference: reproduced to the bit."""
-    if not _have_reference():
-        pytest.skip("reference tree not present (GPU box): pinned by the stored fixtures instead")
     from fuzz_cases import random_big_scene
-    from oracle.harness import Ref, Oracle, ORACLE_STREAM
     _, scene, s = random_big_scene(seed)
-    r = Ref(mocap=False)
-    r.reset()
-    r.load(scene)
-    r.set_settings(s)
-    r.rng(1, s.seed, 0)
-    ref_img, ref_ab, _ = r.render_loop(int(s.frame), reset_policy=1, seed=s.seed)
-    img, ab, _, _ = Oracle(scene).render(s, mode=ORACLE_STREAM)
-    assert (ab == ref_ab).all(), (seed, "abort masks differ")
-    assert np.array_equal(ref_img, img, equal_nan=True), (seed, float(np.nanmax(np.abs(ref_img - img))))
+    _pinned_render(f"big_random_scenes/{seed}", scene, s)
 
 
 @pytest.mark.parametrize("seed", range(4))
 def test_restatement_matches_reference_with_the_cloud_background(oracle_lib, seed):
     """fuzz_cases.sky_case: mutated fixture scenes in front of the value-noise clouds (perlin_cloud: cloudColor per missed
     sample, noise.h) loaded INTO the compiled reference: reproduced to the bit."""
-    if not _have_reference():
-        pytest.skip("reference tree not present (GPU box): pinned by the stored fixtures instead")
     from fuzz_cases import sky_case
-    from oracle.harness import Ref, Oracle, ORACLE_STREAM
     _, scene, s = sky_case(seed)
-    r = Ref(mocap=False)
-    r.reset()
-    r.load(scene)
-    r.set_settings(s)
-    r.rng(1, s.seed, 0)
-    ref_img, ref_ab, _ = r.render_loop(int(s.frame), reset_policy=1, seed=s.seed)
-    img, ab, _, _ = Oracle(scene).render(s, mode=ORACLE_STREAM)
-    assert (ab == ref_ab).all(), (seed, "abort masks differ")
-    assert np.array_equal(ref_img, img, equal_nan=True), (seed, float(np.nanmax(np.abs(ref_img - img))))
+    _pinned_render(f"cloud_background/{seed}", scene, s)
 
 
 @pytest.mark.parametrize("cfg", ["config1", "config2", "config3"])
@@ -187,27 +172,19 @@ def test_restatement_matches_reference_on_the_bench_workloads(oracle_lib, cfg):
     triangles, rectangle light, glossy floor, DOF) loaded INTO the compiled reference at reduced size: the restatement
     reproduces the reference's image to the bit -- except where the reference's own result is undefined (glass, Q3).  (Configs 4 and 5 use per-primitive velocities / a mesh type, which the
     reference does not have; their oracle paths are the same code driven by other inputs.)"""
-    if not _have_reference():
-        pytest.skip("reference tree not present (GPU box): pinned by the stored fixtures instead")
     from distraytracer_b200 import scenes
-    from oracle.harness import Ref, Oracle, ORACLE_STREAM
+    from oracle.harness import Oracle, ORACLE_STREAM
     scene, s = {"config1": scenes.config1, "config2": lambda: scenes.config2(64, 36, 4),
                 "config3": lambda: scenes.config3(64, 36, 4)}[cfg]()
     if cfg == "config1":
         s.xRes, s.yRes = 64, 48
     s.seed = 4242
-    r = Ref(mocap=True)
-    r.reset()
-    r.load(scene)
-    r.set_settings(s)
-    r.rng(1, s.seed, 0)
-    ref_img, ref_ab, _ = r.render_loop(s.frame, reset_policy=1, seed=s.seed)
+    if cfg != "config2":
+        img, _, cnt = _pinned_render(f"bench_workloads/{cfg}", scene, s, mocap=True)
+        assert np.nanstd(img) > 5 and cnt.rays > s.xRes * s.yRes
+        return
     img, ab, cnt, _ = Oracle(scene).render(s, mode=ORACLE_STREAM)
     assert np.nanstd(img) > 5 and cnt.rays > s.xRes * s.yRes
-    same = (ab == ref_ab) & (np.nan_to_num(ref_img, nan=-1.0) == np.nan_to_num(img, nan=-1.0)).all(axis=-1)
-    if cfg != "config2":
-        assert same.all()
-        return
     # config 2 holds glass.  Where a ray tree reaches a glass surface the reference reads an UNINITIALISED variable
     # (`inside = inside_tmp`, render_final_project.cpp:524,534 -- quirk Q3): what it renders there depends on the compiler, and
     # the restatement implements the evident intent (the inside flag of the closest hit).  Everywhere else: to the bit.
@@ -230,15 +207,19 @@ def test_restatement_matches_reference_on_the_bench_workloads(oracle_lib, cfg):
     for dy in (-1, 0, 1):
         for dx in (-1, 0, 1):
             grown |= np.roll(np.roll(touches_glass, dy, axis=0), dx, axis=1)
-    assert same[~grown].all()
-    assert 0 < grown.mean() < 0.25 and 0 < (~same).sum() <= grown.sum()
-    # and with the glass taken out of the material the whole frame is bit-identical again
-    r.reset()
-    r.load(Scene(plain, scene.lights, scene.textures))
-    r.set_settings(s)
-    r.rng(1, s.seed, 0)
-    ref2, ref2_ab, _ = r.render_loop(s.frame, reset_policy=1, seed=s.seed)
-    assert (ref2_ab == nab).all() and np.array_equal(ref2, no_glass, equal_nan=True)
+    assert 0 < grown.mean() < 0.25
+    live = _have_reference()
+    if live:
+        ref_img, ref_ab = _reference_render(scene, s, mocap=True)
+        same = (ab == ref_ab) & (np.nan_to_num(ref_img, nan=-1.0) == np.nan_to_num(img, nan=-1.0)).all(axis=-1)
+        assert same[~grown].all()
+        assert 0 < (~same).sum() <= grown.sum()
+        # and with the glass taken out of the material the whole frame is bit-identical again
+        ref2, ref2_ab = _reference_render(Scene(plain, scene.lights, scene.textures), s, mocap=True)
+        assert (ref2_ab == nab).all() and np.array_equal(ref2, no_glass, equal_nan=True)
+    assert_pinned("bench_workloads/config2/outside_glass", np.where(grown[..., None], np.float32(0), img), ab & ~grown,
+                  matched_reference=live)
+    assert_pinned("bench_workloads/config2/glass_as_plain_surfaces", no_glass, nab, matched_reference=live)
 
 
 def test_restatement_matches_reference_on_a_textured_triangle_terrain(oracle_lib):
@@ -246,11 +227,8 @@ def test_restatement_matches_reference_on_a_textured_triangle_terrain(oracle_lib
     DOF), its mesh handed to the reference as individual Triangle primitives (what its loadObj path produces) and run
     through the reference's own SAH BVH: the restatement reproduces it to the bit.  The velocity blur of config 5 is
     switched off -- the reference has no per-primitive velocities."""
-    if not _have_reference():
-        pytest.skip("reference tree not present (GPU box): pinned by the stored fixtures instead")
     from distraytracer_b200 import scenes, abi
     from distraytracer_b200.scene import Scene
-    from oracle.harness import Ref, Oracle, ORACLE_STREAM
     scene, s = scenes.config5(n=12, xres=64, yres=36, spp=4)
     s.blur_samples, s.blur_mode, s.seed = 0, abi.BLUR_REFERENCE, 777
     prims = [abi.copy_struct(p) for p in scene.prims]
@@ -258,15 +236,7 @@ def test_restatement_matches_reference_on_a_textured_triangle_terrain(oracle_lib
         p.flags &= ~abi.FLAG_MOTION
         p.velocity[:] = [0.0, 0.0, 0.0]
     flat = Scene(prims + scenes.mesh_to_prims(scene.mesh), scene.lights, scene.textures)
-    r = Ref(mocap=True)
-    r.reset()
-    r.load(flat)
-    r.set_settings(s)
-    r.rng(1, s.seed, 0)
-    ref_img, ref_ab, _ = r.render_loop(s.frame, reset_policy=1, seed=s.seed)
-    img, ab, cnt, _ = Oracle(flat).render(s, mode=ORACLE_STREAM)
-    assert (ab == ref_ab).all()
-    assert np.array_equal(ref_img, img, equal_nan=True), float(np.nanmax(np.abs(ref_img - img)))
+    img, _, cnt = _pinned_render("textured_triangle_terrain", flat, s, mocap=True)
     assert np.nanstd(img) > 5 and cnt.prim_tests[abi.PRIM_TRIANGLE] > 0
 
 
