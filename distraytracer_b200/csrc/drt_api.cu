@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "../../include/drt.h"
+#include "drt_box.cuh"
 #include "drt_launch.h"
 #include "drt_bvh_order.h"
 #include "drt_mesh.h"
@@ -136,6 +137,105 @@ void primBounds(const drt_prim& p, double lo[3], double hi[3]) {
   }
 }
 
+// the flattener's replay of the reference's BVH build over the primitives (drt_bvh_order.h)
+ReferenceBVH referenceBVH(const drt_prim* prims, int n_prims) {
+  std::vector<double> centers(3 * (size_t)n_prims);
+  for (int i = 0; i < n_prims; i++) for (int a = 0; a < 3; a++) centers[3 * i + a] = prims[i].center[a];
+  ReferenceBVH bvh;
+  bvh.build(centers.data(), n_prims, [&](int prim, double lo[3], double hi[3]) { primBounds(prims[prim], lo, hi); });
+  return bvh;
+}
+
+// Slab-filter table (drt_kernels.cuh: slabMask) over the padded fp32 boxes of the geoms: one pair record (drt_box.cuh) per
+// two geoms, padded to whole groups of 8 geoms (slabPairWords), then one box per group {cx cy cz hx} {hy hz - -}.  Holes
+// and the padding entries are empty so that they never pass.
+template <typename R>
+std::vector<float4> slabTable(const std::vector<Geom<R>>& geoms) {
+  const size_t n_pairs = 4 * ((geoms.size() + 7) / 8);
+  std::vector<float4> t(3 * n_pairs);
+  for (size_t p = 0; p < n_pairs; p++) {
+    float c[2][3], h[2][3];
+    for (int k = 0; k < 2; k++) {
+      const size_t gi = 2 * p + k;
+      const bool live = gi < geoms.size() && geoms[gi].type != G_HOLE;
+      for (int a = 0; a < 3; a++) {
+        if (live) centreHalf((&geoms[gi].blo.x)[a], (&geoms[gi].bhi.x)[a], c[k][a], h[k][a]);
+        else { c[k][a] = 0.f; h[k][a] = kEmptyHalf; }
+      }
+    }
+    packPair(&t[3 * p], c[0], h[0], c[1], h[1]);
+  }
+  for (size_t g0 = 0; g0 < geoms.size(); g0 += 8) {
+    float lo[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, hi[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
+    bool any = false;
+    for (size_t gi = g0; gi < std::min(geoms.size(), g0 + 8); gi++) {
+      if (geoms[gi].type == G_HOLE) continue;
+      any = true;
+      for (int a = 0; a < 3; a++) { lo[a] = std::min(lo[a], (&geoms[gi].blo.x)[a]); hi[a] = std::max(hi[a], (&geoms[gi].bhi.x)[a]); }
+    }
+    float c[3], h[3];
+    for (int a = 0; a < 3; a++) {
+      if (!any) { c[a] = 0.f; h[a] = kEmptyHalf; continue; }
+      centreHalf(lo[a], hi[a], c[a], h[a]);
+      h[a] = nextafterf(h[a], INFINITY) * 1.000001f;   // also covers the members' own rounded-up half-extents
+    }
+    t.push_back(make_float4(c[0], c[1], c[2], h[0]));
+    t.push_back(make_float4(h[1], h[2], 0.f, 0.f));
+  }
+  return t;
+}
+
+// For scenes with more geoms than the shared-memory table holds: a 4-wide tree (drt_box.cuh) over the geoms, so that
+// closestHit / anyHit gather candidates in O(log n) instead of running the filter over all n.  Median splits of the box
+// centres along the widest axis, twice per node; leaf = one geom (reference -(geom + 1)); node 0 is the root.  Empty when
+// not built: below that size, and when a slab-box prism is present (its intersectShadow can throw, and which pixels then
+// abort depends on the reference's candidate ORDER, which only the linear walk keeps).
+template <typename R>
+std::vector<float4> geomTree(const std::vector<Geom<R>>& geoms) {
+  std::vector<float4> tree;
+  std::vector<int> items;
+  bool any_box = false;
+  for (size_t gi = 0; gi < geoms.size(); gi++) {
+    if (geoms[gi].type == G_BOX) any_box = true;
+    if (geoms[gi].type != G_HOLE) items.push_back((int)gi);
+  }
+  if ((int)geoms.size() <= DRT_SMEM_GEOMS || any_box || items.size() < 2) return tree;
+  auto centre = [&](int gi, int a) { return 0.5f * ((&geoms[gi].blo.x)[a] + (&geoms[gi].bhi.x)[a]); };
+  auto halve = [&](int* first, int* last) {            // median split along the widest axis of the box centres
+    float lo[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, hi[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
+    for (int* it = first; it != last; ++it) for (int a = 0; a < 3; a++) { lo[a] = std::min(lo[a], centre(*it, a)); hi[a] = std::max(hi[a], centre(*it, a)); }
+    int ax = 0; for (int a = 1; a < 3; a++) if (hi[a] - lo[a] > hi[ax] - lo[ax]) ax = a;
+    int* mid = first + (last - first) / 2;
+    std::nth_element(first, mid, last, [&](int x, int y) { const float cx = centre(x, ax), cy = centre(y, ax); return cx < cy || (cx == cy && x < y); });
+    return mid;
+  };
+  // iterative build: a work list of (node index, item range)
+  struct Work { int node; int* first; int* last; };
+  std::vector<Work> work;
+  tree.resize(8);
+  work.push_back({0, items.data(), items.data() + items.size()});
+  while (!work.empty()) {
+    const Work w = work.back(); work.pop_back();
+    int* cuts[5] = {w.first, nullptr, nullptr, nullptr, w.last};
+    cuts[2] = halve(w.first, w.last);
+    cuts[1] = (cuts[2] - cuts[0] >= 2) ? halve(cuts[0], cuts[2]) : cuts[0];
+    cuts[3] = (cuts[4] - cuts[2] >= 2) ? halve(cuts[2], cuts[4]) : cuts[2];
+    float cc[4][3], hh[4][3]; int ref[4]; int m = 0;
+    for (int k = 0; k < 4; k++) {
+      if (cuts[k + 1] == cuts[k]) continue;
+      float lo[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, hi[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
+      for (const int* it = cuts[k]; it != cuts[k + 1]; ++it)
+        for (int a = 0; a < 3; a++) { lo[a] = std::min(lo[a], (&geoms[*it].blo.x)[a]); hi[a] = std::max(hi[a], (&geoms[*it].bhi.x)[a]); }
+      for (int a = 0; a < 3; a++) centreHalf(lo[a], hi[a], cc[m][a], hh[m][a]);
+      if (cuts[k + 1] - cuts[k] == 1) ref[m] = -(*cuts[k] + 1);
+      else { ref[m] = (int)(tree.size() / 8); tree.resize(tree.size() + 8); work.push_back({ref[m], cuts[k], cuts[k + 1]}); }
+      m++;
+    }
+    packNode4(tree.data() + 8 * (size_t)w.node, m, cc, hh, ref);
+  }
+  return tree;
+}
+
 template <typename R>
 struct HostScene {
   std::vector<NodeD<R>> nodes;
@@ -152,10 +252,7 @@ int flatten(const drt_prim* prims, int n_prims, const drt_light* lights, int n_l
   hs.prims.assign(n_prims, PrimD<R>());
   // geoms are emitted in the reference's candidate order so that ties of t between
   // coplanar shapes resolve to the same shape (see drt_bvh_order.h)
-  std::vector<double> centers(3 * (size_t)n_prims);
-  for (int i = 0; i < n_prims; i++) for (int a = 0; a < 3; a++) centers[3 * i + a] = prims[i].center[a];
-  ReferenceBVH bvh;
-  bvh.build(centers.data(), n_prims, [&](int prim, double lo[3], double hi[3]) { primBounds(prims[prim], lo, hi); });
+  const ReferenceBVH bvh = referenceBVH(prims, n_prims);
   const std::vector<int>& order = bvh.order;
   std::vector<int> geom_start(n_prims + 1, 0);   // first geom of the oi-th primitive in reference order
   for (int oi = 0; oi < n_prims; oi++) {
@@ -203,8 +300,6 @@ int flatten(const drt_prim* prims, int n_prims, const drt_light* lights, int n_l
         D3 axis = normalized(c2 - c1);                                   // geometry.cpp:231
         q.pA = cv<R>(c1); q.pG = cv<R>(axis); q.axis_norm = (float)norm(axis);
         if (p.type == DRT_PRIM_CHECKER_CYLINDER) objMatrix<R>(q.objM, axis, c1);
-        if ((p.flags & DRT_FLAG_VERTEX_MOTION) && p.type != DRT_PRIM_CYLINDER)
-          return fail(DRT_ERR_UNSUPPORTED, "DRT_FLAG_VERTEX_MOTION: cylinders only");
         if (p.flags & DRT_FLAG_VERTEX_MOTION) { q.n1 = cv<R>(c2); q.n2 = cv<R>(V(p.velocity2)); }   // see PrimD::vel
         Geom<R> g; memset(&g, 0, sizeof(g));
         g.type = G_CYL; g.owner = i; g.p0 = cv<R>(c1); g.p1 = cv<R>(c2); g.p2 = cv<R>(axis); g.f0 = (float)p.radius; g.vel = cv<R>(vel);
@@ -326,123 +421,10 @@ int flatten(const drt_prim* prims, int n_prims, const drt_light* lights, int n_l
     if (rn.leaf) { nd.first = geom_start[rn.first]; nd.count = geom_start[rn.first + rn.count] - nd.first; }
     hs.nodes.push_back(nd);
   }
-  // slab-filter table (drt_kernels.cuh: slabMask): centre / half-extent of the padded fp32 boxes, two geoms per
-  // record of three float4 {cx0 cx1 cy0 cy1} {cz0 cz1 hx0 hx1} {hy0 hy1 hz0 hz1}, padded to whole groups of 8 geoms
-  // (slabPairWords); holes and the padding entries get a negative half-extent so that they never pass
-  hs.gbounds.clear();
-  for (size_t p = 0; p < 4 * ((hs.geoms.size() + 7) / 8); p++) {
-    float c[2][3], h[2][3];
-    for (int k = 0; k < 2; k++) {
-      const size_t gi = 2 * p + k;
-      const bool live = gi < hs.geoms.size() && hs.geoms[gi].type != G_HOLE;
-      for (int a = 0; a < 3; a++) {
-        if (!live) { c[k][a] = 0.f; h[k][a] = -1e30f; continue; }
-        const float lo = (&hs.geoms[gi].blo.x)[a], hi = (&hs.geoms[gi].bhi.x)[a];
-        const float cf = (float)(0.5 * ((double)lo + (double)hi));
-        const double hd = std::max((double)hi - (double)cf, (double)cf - (double)lo);
-        float hf = (float)hd;
-        if ((double)hf < hd) hf = nextafterf(hf, INFINITY);
-        c[k][a] = cf; h[k][a] = nextafterf(hf, INFINITY);              // [c - h, c + h] contains [lo, hi]
-      }
-    }
-    hs.gbounds.push_back(make_float4(c[0][0], c[1][0], c[0][1], c[1][1]));
-    hs.gbounds.push_back(make_float4(c[0][2], c[1][2], h[0][0], h[1][0]));
-    hs.gbounds.push_back(make_float4(h[0][1], h[1][1], h[0][2], h[1][2]));
-  }
-  // ... followed by one box per group of 8 consecutive geoms: {cx cy cz hx} {hy hz - -}
-  for (size_t g0 = 0; g0 < hs.geoms.size(); g0 += 8) {
-    float lo[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, hi[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
-    bool any = false;
-    for (size_t gi = g0; gi < std::min(hs.geoms.size(), g0 + 8); gi++) {
-      if (hs.geoms[gi].type == G_HOLE) continue;
-      any = true;
-      for (int a = 0; a < 3; a++) { lo[a] = std::min(lo[a], (&hs.geoms[gi].blo.x)[a]); hi[a] = std::max(hi[a], (&hs.geoms[gi].bhi.x)[a]); }
-    }
-    float c[3], h[3];
-    for (int a = 0; a < 3; a++) {
-      if (!any) { c[a] = 0.f; h[a] = -1e30f; continue; }
-      c[a] = (float)(0.5 * ((double)lo[a] + (double)hi[a]));
-      const double hd = std::max((double)hi[a] - (double)c[a], (double)c[a] - (double)lo[a]);
-      float hf = (float)hd;
-      if ((double)hf < hd) hf = nextafterf(hf, INFINITY);
-      h[a] = nextafterf(nextafterf(hf, INFINITY), INFINITY) * 1.000001f;   // also covers the members' own rounded-up half-extents
-    }
-    hs.gbounds.push_back(make_float4(c[0], c[1], c[2], h[0]));
-    hs.gbounds.push_back(make_float4(h[1], h[2], 0.f, 0.f));
-  }
-  // ... and, for scenes with more geoms than the shared-memory table holds, by a 4-wide tree over the geoms in the node
-  // format of the mesh LBVH (drt_lbvh.cuh): closestHit / anyHit then gather candidates in O(log n) instead of running the
-  // filter over all n.  Median splits of the box centres along the widest axis, twice per node; leaf = one geom
-  // (reference -(geom + 1)).  Not built when a slab-box prism is present: its intersectShadow can throw, and which
-  // pixels then abort depends on the reference's candidate ORDER, which only the linear walk keeps.
-  hs.geom_tree = -1;
-  {
-    std::vector<int> items;
-    bool any_box = false;
-    for (size_t gi = 0; gi < hs.geoms.size(); gi++) {
-      if (hs.geoms[gi].type == G_BOX) any_box = true;
-      if (hs.geoms[gi].type != G_HOLE) items.push_back((int)gi);
-    }
-    if ((int)hs.geoms.size() > DRT_SMEM_GEOMS && !any_box && items.size() >= 2) {
-      struct Box { float lo[3], hi[3]; };
-      auto boxOf = [&](const int* first, const int* last) {
-        Box b; for (int a = 0; a < 3; a++) { b.lo[a] = FLT_MAX; b.hi[a] = -FLT_MAX; }
-        for (const int* it = first; it != last; ++it)
-          for (int a = 0; a < 3; a++) { b.lo[a] = std::min(b.lo[a], (&hs.geoms[*it].blo.x)[a]); b.hi[a] = std::max(b.hi[a], (&hs.geoms[*it].bhi.x)[a]); }
-        return b;
-      };
-      auto halve = [&](int* first, int* last) {            // median split along the widest axis of the box centres
-        float lo[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, hi[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
-        auto centre = [&](int gi, int a) { return 0.5f * ((&hs.geoms[gi].blo.x)[a] + (&hs.geoms[gi].bhi.x)[a]); };
-        for (int* it = first; it != last; ++it) for (int a = 0; a < 3; a++) { lo[a] = std::min(lo[a], centre(*it, a)); hi[a] = std::max(hi[a], centre(*it, a)); }
-        int ax = 0; for (int a = 1; a < 3; a++) if (hi[a] - lo[a] > hi[ax] - lo[ax]) ax = a;
-        int* mid = first + (last - first) / 2;
-        std::nth_element(first, mid, last, [&](int x, int y) { const float cx = centre(x, ax), cy = centre(y, ax); return cx < cy || (cx == cy && x < y); });
-        return mid;
-      };
-      const size_t base = hs.gbounds.size();
-      std::vector<float4> tree;
-      // iterative build: a work list of (node index, item range); node 0 is the root
-      struct Work { int node; int* first; int* last; };
-      std::vector<Work> work;
-      tree.resize(8);
-      work.push_back({0, items.data(), items.data() + items.size()});
-      while (!work.empty()) {
-        const Work w = work.back(); work.pop_back();
-        int* cuts[5] = {w.first, nullptr, nullptr, nullptr, w.last};
-        cuts[2] = halve(w.first, w.last);
-        cuts[1] = (cuts[2] - cuts[0] >= 2) ? halve(cuts[0], cuts[2]) : cuts[0];
-        cuts[3] = (cuts[4] - cuts[2] >= 2) ? halve(cuts[2], cuts[4]) : cuts[2];
-        float cc[4][3], hh[4][3]; int ref[4]; int m = 0;
-        for (int k = 0; k < 4; k++) {
-          if (cuts[k + 1] == cuts[k]) continue;
-          const Box b = boxOf(cuts[k], cuts[k + 1]);
-          for (int a = 0; a < 3; a++) {
-            const float cf = (float)(0.5 * ((double)b.lo[a] + (double)b.hi[a]));
-            const double hd = std::max((double)b.hi[a] - (double)cf, (double)cf - (double)b.lo[a]);
-            float hf = (float)hd;
-            if ((double)hf < hd) hf = nextafterf(hf, INFINITY);
-            cc[m][a] = cf; hh[m][a] = nextafterf(hf, INFINITY);
-          }
-          if (cuts[k + 1] - cuts[k] == 1) ref[m] = -(*cuts[k] + 1);
-          else { ref[m] = (int)(tree.size() / 8); tree.resize(tree.size() + 8); work.push_back({ref[m], cuts[k], cuts[k + 1]}); }
-          m++;
-        }
-        for (int k = m; k < 4; k++) { ref[k] = (int)0x80000000; for (int a = 0; a < 3; a++) { cc[k][a] = 0.f; hh[k][a] = -1e30f; } }
-        float4* nd = tree.data() + 8 * (size_t)w.node;
-        for (int p2 = 0; p2 < 2; p2++) {
-          const int a = 2 * p2, b = 2 * p2 + 1;
-          nd[3 * p2 + 0] = make_float4(cc[a][0], cc[b][0], cc[a][1], cc[b][1]);
-          nd[3 * p2 + 1] = make_float4(cc[a][2], cc[b][2], hh[a][0], hh[b][0]);
-          nd[3 * p2 + 2] = make_float4(hh[a][1], hh[b][1], hh[a][2], hh[b][2]);
-        }
-        float4 refs; memcpy(&refs.x, &ref[0], 4); memcpy(&refs.y, &ref[1], 4); memcpy(&refs.z, &ref[2], 4); memcpy(&refs.w, &ref[3], 4);
-        nd[6] = refs; nd[7] = make_float4(0.f, 0.f, 0.f, 0.f);
-      }
-      hs.geom_tree = (int)base;
-      hs.gbounds.insert(hs.gbounds.end(), tree.begin(), tree.end());
-    }
-  }
+  hs.gbounds = slabTable(hs.geoms);
+  const std::vector<float4> tree = geomTree(hs.geoms);
+  hs.geom_tree = tree.empty() ? -1 : (int)hs.gbounds.size();
+  hs.gbounds.insert(hs.gbounds.end(), tree.begin(), tree.end());
   for (size_t k = 0; k < hs.nodes.size(); k++) {
     NodeD<R>& nd = hs.nodes[k];
     if (nd.leaf) { for (int gi = nd.first; gi < nd.first + nd.count; gi++) hs.geoms[gi].leaf = (int)k; }
@@ -475,8 +457,8 @@ int flatten(const drt_prim* prims, int n_prims, const drt_light* lights, int n_l
 
 template <typename R>
 struct DevScene {
-  Geom<R>* geoms = nullptr; PrimD<R>* prims = nullptr; LightD<R>* lights = nullptr; NodeD<R>* nodes = nullptr;
-  float4* gbounds = nullptr; size_t gbounds_words = 0;
+  DevBuf<Geom<R>> geoms; DevBuf<PrimD<R>> prims; DevBuf<LightD<R>> lights; DevBuf<NodeD<R>> nodes;
+  DevBuf<float4> gbounds;
   int geom_tree = -1;       // word offset of the 4-wide tree over the geoms inside gbounds, or -1 (HostScene::geom_tree)
   int n_geoms = 0, n_prims = 0, n_lights = 0, n_nodes = 0;
 };
@@ -515,33 +497,15 @@ size_t uploadBytes(const HostScene<R>& hs) {
 
 template <typename R>
 int upload(const HostScene<R>& hs, DevScene<R>& ds, PinnedStage& stage, cudaStream_t q) {
-  if ((int)hs.geoms.size() != ds.n_geoms || !ds.geoms) {
-    if (ds.geoms) cudaFree(ds.geoms);
-    CK(cudaMalloc(&ds.geoms, sizeof(Geom<R>) * std::max<size_t>(1, hs.geoms.size())));
-  }
-  if (hs.gbounds.size() != ds.gbounds_words || !ds.gbounds) {
-    if (ds.gbounds) cudaFree(ds.gbounds);
-    ds.gbounds = nullptr;
-    CK(cudaMalloc(&ds.gbounds, sizeof(float4) * std::max<size_t>(3, hs.gbounds.size())));
-    ds.gbounds_words = hs.gbounds.size();
-  }
+  CK(ds.gbounds.reserve(sizeof(float4) * std::max<size_t>(3, hs.gbounds.size())));
+  CK(ds.nodes.reserve(sizeof(NodeD<R>) * std::max<size_t>(1, hs.nodes.size())));
+  CK(ds.geoms.reserve(sizeof(Geom<R>) * std::max<size_t>(1, hs.geoms.size())));
+  CK(ds.prims.reserve(sizeof(PrimD<R>) * std::max<size_t>(1, hs.prims.size())));
+  CK(ds.lights.reserve(sizeof(LightD<R>) * std::max<size_t>(1, hs.lights.size())));
   ds.geom_tree = hs.geom_tree;
+  ds.n_nodes = (int)hs.nodes.size(); ds.n_geoms = (int)hs.geoms.size(); ds.n_prims = (int)hs.prims.size(); ds.n_lights = (int)hs.lights.size();
   { int rc = stage.push(ds.gbounds, hs.gbounds.data(), sizeof(float4) * hs.gbounds.size(), q); if (rc) return rc; }
-  if ((int)hs.prims.size() != ds.n_prims || !ds.prims) {
-    if (ds.prims) cudaFree(ds.prims);
-    CK(cudaMalloc(&ds.prims, sizeof(PrimD<R>) * std::max<size_t>(1, hs.prims.size())));
-  }
-  if ((int)hs.lights.size() != ds.n_lights || !ds.lights) {
-    if (ds.lights) cudaFree(ds.lights);
-    CK(cudaMalloc(&ds.lights, sizeof(LightD<R>) * std::max<size_t>(1, hs.lights.size())));
-  }
-  if ((int)hs.nodes.size() != ds.n_nodes || !ds.nodes) {
-    if (ds.nodes) cudaFree(ds.nodes);
-    CK(cudaMalloc(&ds.nodes, sizeof(NodeD<R>) * std::max<size_t>(1, hs.nodes.size())));
-  }
-  ds.n_nodes = (int)hs.nodes.size();
   { int rc = stage.push(ds.nodes, hs.nodes.data(), sizeof(NodeD<R>) * ds.n_nodes, q); if (rc) return rc; }
-  ds.n_geoms = (int)hs.geoms.size(); ds.n_prims = (int)hs.prims.size(); ds.n_lights = (int)hs.lights.size();
   { int rc = stage.push(ds.geoms, hs.geoms.data(), sizeof(Geom<R>) * ds.n_geoms, q); if (rc) return rc; }
   { int rc = stage.push(ds.prims, hs.prims.data(), sizeof(PrimD<R>) * ds.n_prims, q); if (rc) return rc; }
   { int rc = stage.push(ds.lights, hs.lights.data(), sizeof(LightD<R>) * ds.n_lights, q); if (rc) return rc; }
@@ -570,17 +534,17 @@ struct drt_scene {
   bool any_glass = false, any_tex = false, any_motion = false, any_box = false, any_spill = false;
   DevScene<double> dd; DevScene<float> df;
   std::vector<cudaArray_t> tex_arrays; std::vector<cudaTextureObject_t> tex_objs;
-  cudaTextureObject_t* d_tex = nullptr; int2* d_texdims = nullptr;
+  DevBuf<cudaTextureObject_t> d_tex; DevBuf<int2> d_texdims;
   cudaStream_t stream = nullptr; cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   // scratch, grown on demand
-  float4* samples = nullptr; size_t samples_cap = 0;
-  unsigned char* need = nullptr; float4* bg = nullptr; size_t corner_cap = 0;
-  unsigned char* out_u8 = nullptr; float* out_f32 = nullptr; size_t out_cap = 0;
-  Counts* counts = nullptr;
-  void* pool = nullptr; size_t pool_cap = 0;
-  unsigned long long* batch_counter = nullptr; int* overflow = nullptr;
-  unsigned long long* steal_counters = nullptr;                 // drt_render_multi: one counter per row chunk, claimed by every device
-  unsigned char* owned = nullptr; size_t owned_cap = 0;         // drt_render_multi: units of the current chunk this device rendered
+  DevBuf<float4> samples;
+  DevBuf<unsigned char> need; DevBuf<float4> bg;
+  DevBuf<unsigned char> out_u8; DevBuf<float> out_f32;
+  DevBuf<Counts> counts;
+  DevBuf<char> pool;
+  DevBuf<unsigned long long> batch_counter; DevBuf<int> overflow;
+  DevBuf<unsigned long long> steal_counters;                    // drt_render_multi: one counter per row chunk, claimed by every device
+  DevBuf<unsigned char> owned;                                  // drt_render_multi: units of the current chunk this device rendered
   cudaEvent_t ev_sync = nullptr;                                // cross-device ordering (drt_render_multi)
   int wave_blocks_f64 = 0, wave_blocks_f32 = 0;
   MeshBuffers mesh; bool has_mesh = false;
@@ -693,7 +657,7 @@ void fillParams(Params<R>& P, const drt_scene* s, const DevScene<R>& ds, const d
   P.tex = s->d_tex; P.texdims = s->d_texdims;
   if (s->has_mesh) {
     P.mesh_nodes = s->mesh.nodes; P.n_mesh_tris = s->mesh.n_tris; P.mesh_prim = (int)s->prims.size();
-    P.mesh_tris = (const MeshTri<R>*)(sizeof(R) == 8 ? s->mesh.tris_f64 : s->mesh.tris_f32);
+    if constexpr (sizeof(R) == 8) P.mesh_tris = s->mesh.tris_f64; else P.mesh_tris = s->mesh.tris_f32;
     P.mesh_mat = s->mesh.mat_ids;
     const drt_prim& m0 = s->mesh_materials[0];
     P.mesh_vel = mk<R>((R)m0.velocity[0], (R)m0.velocity[1], (R)m0.velocity[2]);
@@ -701,31 +665,14 @@ void fillParams(Params<R>& P, const drt_scene* s, const DevScene<R>& ds, const d
 }
 
 int ensureScratch(drt_scene* s, size_t n_samples, size_t n_corners, size_t n_out) {
-  if (n_samples > s->samples_cap) {
-    if (s->samples) cudaFree(s->samples);
-    s->samples = nullptr; s->samples_cap = 0;
-    CK(cudaMalloc(&s->samples, n_samples * sizeof(float4)));
-    s->samples_cap = n_samples;
-  }
-  if (n_corners > s->corner_cap) {
-    if (s->need) cudaFree(s->need);
-    if (s->bg) cudaFree(s->bg);
-    s->need = nullptr; s->bg = nullptr; s->corner_cap = 0;
-    CK(cudaMalloc(&s->need, n_corners));
-    CK(cudaMalloc(&s->bg, n_corners * sizeof(float4)));
-    s->corner_cap = n_corners;
-  }
-  if (n_out > s->out_cap) {
-    if (s->out_u8) cudaFree(s->out_u8);
-    if (s->out_f32) cudaFree(s->out_f32);
-    s->out_u8 = nullptr; s->out_f32 = nullptr; s->out_cap = 0;
-    CK(cudaMalloc(&s->out_u8, n_out));
-    CK(cudaMalloc(&s->out_f32, n_out * sizeof(float)));
-    s->out_cap = n_out;
-  }
-  if (!s->counts) CK(cudaMalloc(&s->counts, sizeof(Counts)));
-  if (!s->batch_counter) CK(cudaMalloc(&s->batch_counter, sizeof(unsigned long long)));
-  if (!s->overflow) { CK(cudaMalloc(&s->overflow, sizeof(int))); CK(cudaMemsetAsync(s->overflow, 0, sizeof(int), s->stream)); }
+  CK(s->samples.reserve(n_samples * sizeof(float4)));
+  CK(s->need.reserve(n_corners));
+  CK(s->bg.reserve(n_corners * sizeof(float4)));
+  CK(s->out_u8.reserve(n_out));
+  CK(s->out_f32.reserve(n_out * sizeof(float)));
+  CK(s->counts.reserve(sizeof(Counts)));
+  CK(s->batch_counter.reserve(sizeof(unsigned long long)));
+  if (!s->overflow) { CK(s->overflow.reserve(sizeof(int))); CK(cudaMemsetAsync(s->overflow, 0, sizeof(int), s->stream)); }
   return DRT_OK;
 }
 
@@ -749,34 +696,40 @@ struct MultiCtx {
 
 // What one render call launches on one scene handle, split into stages so that drt_render_multi can interleave the
 // stages of several handles: plan (allocations, kernel parameters) -> per row chunk: render, background, resolve.
+template <typename R>
 struct LaunchPlan {
-  bool f32 = false;
-  Params<double> Pd; Params<float> Pf;
+  Params<R> P;
   bool collect = false, perlin = false, cloud_only = false;
   int tile_h = 0, rows_per_chunk = 1, n_chunks = 1;
   long long per_row = 0;
   size_t n_corners = 0;
   int feat = 0, wave_blocks = 0, launches = 0, variant = -1;
 };
-template <typename R> Params<R>& planParams(LaunchPlan& lp);
-template <> Params<double>& planParams<double>(LaunchPlan& lp) { return lp.Pd; }
-template <> Params<float>& planParams<float>(LaunchPlan& lp) { return lp.Pf; }
+
+template <typename R> const DevScene<R>& devScene(const drt_scene* s) { if constexpr (sizeof(R) == 8) return s->dd; else return s->df; }
+
+// Camera samples per tile row, and rows per render launch: as many as fit maxChunkSamples(), at least one (the whole tile
+// for cloud_only frames, which render no samples)
+void chunking(const drt_settings& st, const drt_tile& tile, long long& per_row, int& rows_per_chunk) {
+  const int n = (int)sqrt((double)st.antialias_samples);
+  per_row = (long long)tile.width * (n * n);
+  rows_per_chunk = st.cloud_only ? tile.height : (int)std::max<long long>(1, std::min<long long>(tile.height, maxChunkSamples() / std::max<long long>(1, per_row)));
+}
 
 template <typename R>
-int planLaunch(drt_scene* s, const DevScene<R>& ds, const drt_settings& st, const CameraD& cam, const drt_tile& tile, int pool_cap,
-               bool want_f32, drt_counters* counters, const MultiCtx* mc, LaunchPlan& lp) {
-  Params<R>& P = planParams<R>(lp);
-  lp.f32 = sizeof(R) == 4;
+int planLaunch(drt_scene* s, const drt_settings& st, const CameraD& cam, const drt_tile& tile, int pool_cap, bool want_f32,
+               drt_counters* counters, const MultiCtx* mc, LaunchPlan<R>& lp) {
+  const DevScene<R>& ds = devScene<R>(s);
+  Params<R>& P = lp.P;
   fillParams<R>(P, s, ds, st, cam, tile);
   lp.collect = counters && counters->collect;
   lp.perlin = st.perlin_cloud && !st.cloud_only; lp.cloud_only = st.cloud_only; lp.tile_h = tile.height;
-  lp.per_row = (long long)tile.width * P.spp;
-  lp.rows_per_chunk = st.cloud_only ? tile.height : (int)std::max<long long>(1, std::min<long long>(tile.height, maxChunkSamples() / std::max<long long>(1, lp.per_row)));
+  chunking(st, tile, lp.per_row, lp.rows_per_chunk);
   lp.n_chunks = (tile.height + lp.rows_per_chunk - 1) / lp.rows_per_chunk;
   lp.n_corners = (size_t)(tile.width + 1) * (tile.height + 1);
   int rc = ensureScratch(s, st.cloud_only ? 1 : (size_t)lp.rows_per_chunk * lp.per_row, lp.n_corners, (size_t)tile.width * tile.height * 3);
   if (rc) return rc;
-  P.samples = s->samples; P.need = s->need; P.bg = s->bg; P.out_u8 = s->out_u8; P.out_f32 = want_f32 ? s->out_f32 : nullptr;
+  P.samples = s->samples; P.need = s->need; P.bg = s->bg; P.out_u8 = s->out_u8; P.out_f32 = want_f32 ? s->out_f32.p : nullptr;
   // claim units: one batch on a single device; whole pixels (at least one batch's worth) when devices share the frame
   P.unit_samples = DRT_CTA_SLOTS;
   if (mc) {
@@ -784,28 +737,16 @@ int planLaunch(drt_scene* s, const DevScene<R>& ds, const drt_settings& st, cons
     P.unit_samples = unit_pixels * P.spp;
     const size_t n_units = ((size_t)lp.rows_per_chunk * lp.per_row + P.unit_samples - 1) / P.unit_samples;
     if (lp.n_chunks > DRT_MULTI_MAX_CHUNKS) return fail(DRT_ERR_UNSUPPORTED, "frame cut into too many row chunks");
-    if (n_units > s->owned_cap) {
-      if (s->owned) cudaFree(s->owned);
-      s->owned = nullptr; s->owned_cap = 0;
-      CK(cudaMalloc(&s->owned, n_units));
-      s->owned_cap = n_units;
-    }
+    CK(s->owned.reserve(n_units));
     P.steal = 1; P.owned = s->owned; P.out_u8 = mc->gather_u8; P.out_f32 = nullptr;
   }
-  P.counts = lp.collect ? s->counts : nullptr;
+  P.counts = lp.collect ? s->counts.p : nullptr;
   int& wave_blocks = sizeof(R) == 8 ? s->wave_blocks_f64 : s->wave_blocks_f32;
   if (!wave_blocks) wave_blocks = waveGridBlocks<R>();
   lp.wave_blocks = wave_blocks;
-  const size_t pool_bytes = wavePoolBytes<R>(wave_blocks, pool_cap);
-  if (!st.cloud_only && pool_bytes > s->pool_cap) {
-    if (s->pool) cudaFree(s->pool);
-    s->pool = nullptr; s->pool_cap = 0;
-    if (cudaMalloc(&s->pool, pool_bytes) != cudaSuccess) {
-      cudaGetLastError();
-      s->pool = nullptr;
-      return fail(DRT_ERR_CUDA, "out of device memory for the ray pools (brdf_samples * max_depth too large)");
-    }
-    s->pool_cap = pool_bytes;
+  if (!st.cloud_only && s->pool.reserve(wavePoolBytes<R>(wave_blocks, pool_cap)) != cudaSuccess) {
+    cudaGetLastError();
+    return fail(DRT_ERR_CUDA, "out of device memory for the ray pools (brdf_samples * max_depth too large)");
   }
   P.pool_raw = s->pool; P.pool_cap = pool_cap; P.batch_counter = s->batch_counter; P.overflow = s->overflow;
   // what this call can reach decides the render_wave instantiation (drt_launch.h WaveFeat)
@@ -823,7 +764,8 @@ int planLaunch(drt_scene* s, const DevScene<R>& ds, const drt_settings& st, cons
 }
 
 // first launches of a call: counters, timing start, background map reset
-int stageBegin(drt_scene* s, LaunchPlan& lp) {
+template <typename R>
+int stageBegin(drt_scene* s, LaunchPlan<R>& lp) {
   cudaStream_t q = s->stream;
   if (lp.collect) CK(cudaMemsetAsync(s->counts, 0, sizeof(Counts), q));
   CK(cudaEventRecord(s->ev0, q));
@@ -831,8 +773,8 @@ int stageBegin(drt_scene* s, LaunchPlan& lp) {
   return DRT_OK;
 }
 template <typename R>
-int stageRender(drt_scene* s, LaunchPlan& lp, int chunk, const MultiCtx* mc) {
-  Params<R>& P = planParams<R>(lp);
+int stageRender(drt_scene* s, LaunchPlan<R>& lp, int chunk, const MultiCtx* mc) {
+  Params<R>& P = lp.P;
   cudaStream_t q = s->stream;
   const int row0 = chunk * lp.rows_per_chunk, rows = std::min(lp.rows_per_chunk, lp.tile_h - row0);
   P.sample_base = (long long)row0 * lp.per_row;
@@ -847,42 +789,41 @@ int stageRender(drt_scene* s, LaunchPlan& lp, int chunk, const MultiCtx* mc) {
 // background colours of the pixel corners marked so far.  `shared`: the marks and colours live in the gathering device's
 // maps and all devices claim blocks of corners from `corner_counter` there (drt_render_multi).
 template <typename R>
-int stageCloud(drt_scene* s, LaunchPlan& lp, unsigned char* need, float4* bg, unsigned long long* corner_counter) {
-  Params<R> P = planParams<R>(lp);
+int stageCloud(drt_scene* s, LaunchPlan<R>& lp, unsigned char* need, float4* bg, unsigned long long* corner_counter) {
+  Params<R> P = lp.P;
   P.need = need; P.bg = bg; P.corner_counter = corner_counter;
   launchCloudCorners<R>(P, s->stream); lp.launches++;
   return DRT_OK;
 }
 template <typename R>
-int stageResolve(drt_scene* s, LaunchPlan& lp, int chunk) {
-  Params<R>& P = planParams<R>(lp);
+int stageResolve(drt_scene* s, LaunchPlan<R>& lp, int chunk) {
   const int row0 = chunk * lp.rows_per_chunk, rows = std::min(lp.rows_per_chunk, lp.tile_h - row0);
-  launchResolve<R>(P, row0, rows, s->stream); lp.launches++;
+  launchResolve<R>(lp.P, row0, rows, s->stream); lp.launches++;
   return DRT_OK;
 }
-int stageEnd(drt_scene* s, LaunchPlan& lp, drt_counters* counters) {
+template <typename R>
+int stageEnd(drt_scene* s, LaunchPlan<R>& lp, drt_counters* counters) {
   CK(cudaEventRecord(s->ev1, s->stream));
   CK(cudaGetLastError());
   if (counters) { counters->kernel_launches = lp.launches; counters->kernel_variant = lp.variant; }
   return DRT_OK;
 }
-#define DRT_BY_PRECISION(lp, call_d, call_f) ((lp).f32 ? (call_f) : (call_d))
 
 template <typename R>
-int launchAll(drt_scene* s, const DevScene<R>& ds, const drt_settings& st, const CameraD& cam, const drt_tile& tile, int pool_cap,
-              bool want_f32, drt_counters* counters) {
-  LaunchPlan lp;
-  int rc = planLaunch<R>(s, ds, st, cam, tile, pool_cap, want_f32, counters, nullptr, lp);
+int launchAll(drt_scene* s, const drt_settings& st, const CameraD& cam, const drt_tile& tile, int pool_cap, bool want_f32,
+              drt_counters* counters) {
+  LaunchPlan<R> lp;
+  int rc = planLaunch<R>(s, st, cam, tile, pool_cap, want_f32, counters, nullptr, lp);
   if (rc) return rc;
   if ((rc = stageBegin(s, lp))) return rc;
   if (st.cloud_only) {
-    if ((rc = stageCloud<R>(s, lp, s->need, s->bg, nullptr))) return rc;
-    if ((rc = stageResolve<R>(s, lp, 0))) return rc;
+    if ((rc = stageCloud(s, lp, s->need, s->bg, nullptr))) return rc;
+    if ((rc = stageResolve(s, lp, 0))) return rc;
   } else {
     for (int c = 0; c < lp.n_chunks; c++) {
-      if ((rc = stageRender<R>(s, lp, c, nullptr))) return rc;
-      if (lp.perlin && (rc = stageCloud<R>(s, lp, s->need, s->bg, nullptr))) return rc;
-      if ((rc = stageResolve<R>(s, lp, c))) return rc;
+      if ((rc = stageRender(s, lp, c, nullptr))) return rc;
+      if (lp.perlin && (rc = stageCloud(s, lp, s->need, s->bg, nullptr))) return rc;
+      if ((rc = stageResolve(s, lp, c))) return rc;
     }
   }
   return stageEnd(s, lp, counters);
@@ -925,18 +866,17 @@ int planRender(drt_scene* s, const drt_settings* st, const drt_tile* tile, int& 
 
 int launchFor(drt_scene* s, const drt_settings* st, const CameraD& cam, const drt_tile* tile, int pool_cap, bool want_f32,
               drt_counters* counters) {
-  if (st->precision == DRT_PRECISION_FP32) return launchAll<float>(s, s->df, *st, cam, *tile, pool_cap, want_f32, counters);
-  return launchAll<double>(s, s->dd, *st, cam, *tile, pool_cap, want_f32, counters);
+  if (st->precision == DRT_PRECISION_FP32) return launchAll<float>(s, *st, cam, *tile, pool_cap, want_f32, counters);
+  return launchAll<double>(s, *st, cam, *tile, pool_cap, want_f32, counters);
 }
 
 // After the scene's stream has been synchronised: overflow flag, timing, event counters (`hc` already copied back).
-int finishRender(drt_scene* s, const drt_settings* st, drt_counters* counters, const Counts& hc, int overflowed) {
+int finishRender(drt_scene* s, drt_counters* counters, const Counts& hc, int overflowed) {
   if (overflowed) {   // the kernel dropped rays instead of writing past its pool: the frame is not valid
     CK(cudaMemsetAsync(s->overflow, 0, sizeof(int), s->stream));
     CK(cudaStreamSynchronize(s->stream));
     return fail(DRT_ERR_UNSUPPORTED, "a CTA ray pool overflowed (brdf_samples * max_depth beyond the sized bound)");
   }
-  (void)st;
   if (counters) {
     float ms = 0; CK(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
     counters->kernel_ms = ms;
@@ -952,6 +892,17 @@ int finishRender(drt_scene* s, const drt_settings* st, drt_counters* counters, c
     }
   }
   return DRT_OK;
+}
+
+// End of a render call on one scene handle (its device current): event counters and overflow flag back, wait for the
+// scene's stream, finishRender.
+int readBack(drt_scene* s, drt_counters* counters, bool check_overflow) {
+  Counts hc; memset(&hc, 0, sizeof(hc));
+  if (counters && counters->collect) CK(cudaMemcpyAsync(&hc, s->counts, sizeof(Counts), cudaMemcpyDeviceToHost, s->stream));
+  int overflowed = 0;
+  if (check_overflow) CK(cudaMemcpyAsync(&overflowed, s->overflow, sizeof(int), cudaMemcpyDeviceToHost, s->stream));
+  CK(cudaStreamSynchronize(s->stream));
+  return finishRender(s, counters, hc, overflowed);
 }
 
 int renderCommon(const drt_scene* cs, const drt_settings* st, const drt_tile* tile, float* out_f32, uint8_t* out_u8,
@@ -971,13 +922,79 @@ int renderCommon(const drt_scene* cs, const drt_settings* st, const drt_tile* ti
     if (out_u8) CK(cudaMemcpyAsync(out_u8, s->out_u8, n_out, cudaMemcpyDeviceToHost, s->stream));
     if (out_f32) CK(cudaMemcpyAsync(out_f32, s->out_f32, n_out * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
   }
-  Counts hc; memset(&hc, 0, sizeof(hc));
-  const bool collect = counters && counters->collect;
-  if (collect) CK(cudaMemcpyAsync(&hc, s->counts, sizeof(Counts), cudaMemcpyDeviceToHost, s->stream));
-  int overflowed = 0;
-  if (!st->cloud_only) CK(cudaMemcpyAsync(&overflowed, s->overflow, sizeof(int), cudaMemcpyDeviceToHost, s->stream));
-  CK(cudaStreamSynchronize(s->stream));
-  return finishRender(s, st, counters, hc, overflowed);
+  return readBack(s, counters, !st->cloud_only);
+}
+
+// The stages of drt_render_multi on all n handles, interleaved chunk by chunk.
+template <typename R>
+int launchMulti(drt_scene* const* scenes, int n, const drt_settings& st, const CameraD& cam, const drt_tile& tile,
+                const int* pool_cap, drt_counters* counters, const MultiCtx& mc) {
+  drt_scene* g = scenes[0];                                     // the gathering device
+  std::vector<LaunchPlan<R>> plans(n);
+  for (int i = 0; i < n; i++) {
+    drt_scene* s = scenes[i];
+    CK(cudaSetDevice(s->device));
+    if (i) CK(cudaStreamWaitEvent(s->stream, g->ev_sync, 0));
+    drt_tile t = tile; t.device = s->device;
+    int rc = planLaunch<R>(s, st, cam, t, pool_cap[i], false, counters ? &counters[i] : nullptr, &mc, plans[i]);
+    if (rc) return rc;
+    if ((rc = stageBegin(s, plans[i]))) return rc;
+    if (i == 0) CK(cudaEventRecord(g->ev_sync, g->stream));    // ... and the shared background map is reset
+  }
+  // every stream waits for every other stream's work so far (events only: the host does not block)
+  auto barrier = [&]() -> int {
+    for (int i = 0; i < n; i++) { CK(cudaSetDevice(scenes[i]->device)); CK(cudaEventRecord(scenes[i]->ev_sync, scenes[i]->stream)); }
+    for (int i = 0; i < n; i++) {
+      CK(cudaSetDevice(scenes[i]->device));
+      for (int k = 0; k < n; k++) if (k != i) CK(cudaStreamWaitEvent(scenes[i]->stream, scenes[k]->ev_sync, 0));
+    }
+    return DRT_OK;
+  };
+  const LaunchPlan<R>& lp0 = plans[0];
+  for (int c = 0; c < lp0.n_chunks; c++) {
+    for (int i = 0; i < n; i++) {
+      CK(cudaSetDevice(scenes[i]->device));
+      int rc = stageRender(scenes[i], plans[i], c, &mc);
+      if (rc) return rc;
+    }
+    if (lp0.perlin) {
+      // The background of a missed sample is a 200-step noise march per pixel CORNER, shared by the four pixels around it:
+      // with the frame dealt out in small units every device would evaluate the corners of its own pixels, up to 4x the
+      // work.  Instead the devices' corner marks are merged in the gathering device's map, all devices claim blocks of
+      // marked corners from one counter, write the colours there, and pull the finished map back before resolving.
+      int rc;
+      for (int i = 1; i < n; i++) {
+        CK(cudaSetDevice(scenes[i]->device));
+        launchNeedPush(scenes[i]->need, g->need, lp0.n_corners, scenes[i]->stream); plans[i].launches++;
+      }
+      CK(cudaSetDevice(g->device));
+      CK(cudaMemsetAsync(g->steal_counters + DRT_MULTI_MAX_CHUNKS + c, 0, sizeof(unsigned long long), g->stream));
+      if ((rc = barrier())) return rc;
+      for (int i = 0; i < n; i++) {
+        CK(cudaSetDevice(scenes[i]->device));
+        if ((rc = stageCloud(scenes[i], plans[i], g->need, g->bg, g->steal_counters + DRT_MULTI_MAX_CHUNKS + c))) return rc;
+      }
+      if ((rc = barrier())) return rc;
+      for (int i = 1; i < n; i++) {
+        CK(cudaSetDevice(scenes[i]->device));
+        CK(cudaMemcpyAsync(scenes[i]->need, g->need, lp0.n_corners, cudaMemcpyDeviceToDevice, scenes[i]->stream));
+        CK(cudaMemcpyAsync(scenes[i]->bg, g->bg, lp0.n_corners * sizeof(float4), cudaMemcpyDeviceToDevice, scenes[i]->stream));
+      }
+    }
+    for (int i = 0; i < n; i++) {
+      CK(cudaSetDevice(scenes[i]->device));
+      int rc = stageResolve(scenes[i], plans[i], c);
+      if (rc) return rc;
+    }
+    // the next chunk's marks and colours go into the gathering device's maps: its resolve must have read them first
+    if (lp0.perlin && c + 1 < lp0.n_chunks) { int rc = barrier(); if (rc) return rc; }
+  }
+  for (int i = 0; i < n; i++) {
+    CK(cudaSetDevice(scenes[i]->device));
+    int rc = stageEnd(scenes[i], plans[i], counters ? &counters[i] : nullptr);
+    if (rc) return rc;
+  }
+  return DRT_OK;
 }
 
 // One frame on several devices at once (include/drt.h drt_render_multi).
@@ -1006,89 +1023,22 @@ int renderMulti(drt_scene* const* scenes, int n, const drt_settings* st, const d
   CK(cudaSetDevice(g->device));
   const size_t n_out = (size_t)tile->width * tile->height * 3;
   {
-    const int spp = (int)sqrt((double)st->antialias_samples) * (int)sqrt((double)st->antialias_samples);
-    const long long per_row = (long long)tile->width * spp;
-    const int rows_per_chunk = (int)std::max<long long>(1, std::min<long long>(tile->height, maxChunkSamples() / std::max<long long>(1, per_row)));
+    long long per_row; int rows_per_chunk;
+    chunking(*st, *tile, per_row, rows_per_chunk);
     int rc = ensureScratch(g, (size_t)rows_per_chunk * per_row, (size_t)(tile->width + 1) * (tile->height + 1), n_out);
     if (rc) return rc;
   }
   // [0, MAX_CHUNKS): unit counters of the row chunks; [MAX_CHUNKS, 2 MAX_CHUNKS): corner-block counters of the background passes
-  if (!g->steal_counters) CK(cudaMalloc(&g->steal_counters, sizeof(unsigned long long) * 2 * DRT_MULTI_MAX_CHUNKS));
+  CK(g->steal_counters.reserve(sizeof(unsigned long long) * 2 * DRT_MULTI_MAX_CHUNKS));
   CK(cudaMemsetAsync(g->steal_counters, 0, sizeof(unsigned long long) * 2 * DRT_MULTI_MAX_CHUNKS, g->stream));
   for (int i = 0; i < n; i++) if (!scenes[i]->ev_sync) { CK(cudaSetDevice(scenes[i]->device)); CK(cudaEventCreateWithFlags(&scenes[i]->ev_sync, cudaEventDisableTiming)); }
   CK(cudaSetDevice(g->device));
   CK(cudaEventRecord(g->ev_sync, g->stream));                  // counters zeroed, frame buffer allocated
   MultiCtx mc; mc.counters = g->steal_counters; mc.gather_u8 = g->out_u8;
-  std::vector<LaunchPlan> plans(n);
-  for (int i = 0; i < n; i++) {
-    drt_scene* s = scenes[i];
-    CK(cudaSetDevice(s->device));
-    if (i) CK(cudaStreamWaitEvent(s->stream, g->ev_sync, 0));
-    drt_tile t = *tile; t.device = s->device;
-    int rc = (st->precision == DRT_PRECISION_FP32)
-                 ? planLaunch<float>(s, s->df, *st, cam, t, pool_cap[i], false, counters ? &counters[i] : nullptr, &mc, plans[i])
-                 : planLaunch<double>(s, s->dd, *st, cam, t, pool_cap[i], false, counters ? &counters[i] : nullptr, &mc, plans[i]);
-    if (rc) return rc;
-    if ((rc = stageBegin(s, plans[i]))) return rc;
-    if (i == 0) CK(cudaEventRecord(g->ev_sync, g->stream));    // ... and the shared background map is reset
-  }
-  // every stream waits for every other stream's work so far (events only: the host does not block)
-  auto barrier = [&]() -> int {
-    for (int i = 0; i < n; i++) { CK(cudaSetDevice(scenes[i]->device)); CK(cudaEventRecord(scenes[i]->ev_sync, scenes[i]->stream)); }
-    for (int i = 0; i < n; i++) {
-      CK(cudaSetDevice(scenes[i]->device));
-      for (int k = 0; k < n; k++) if (k != i) CK(cudaStreamWaitEvent(scenes[i]->stream, scenes[k]->ev_sync, 0));
-    }
-    return DRT_OK;
-  };
-  const LaunchPlan& lp0 = plans[0];
-  for (int c = 0; c < lp0.n_chunks; c++) {
-    for (int i = 0; i < n; i++) {
-      CK(cudaSetDevice(scenes[i]->device));
-      int rc = DRT_BY_PRECISION(plans[i], stageRender<double>(scenes[i], plans[i], c, &mc), stageRender<float>(scenes[i], plans[i], c, &mc));
-      if (rc) return rc;
-    }
-    if (lp0.perlin) {
-      // The background of a missed sample is a 200-step noise march per pixel CORNER, shared by the four pixels around it:
-      // with the frame dealt out in small units every device would evaluate the corners of its own pixels, up to 4x the
-      // work.  Instead the devices' corner marks are merged in the gathering device's map, all devices claim blocks of
-      // marked corners from one counter, write the colours there, and pull the finished map back before resolving.
-      int rc;
-      for (int i = 1; i < n; i++) {
-        CK(cudaSetDevice(scenes[i]->device));
-        launchNeedPush(scenes[i]->need, g->need, lp0.n_corners, scenes[i]->stream); plans[i].launches++;
-      }
-      CK(cudaSetDevice(g->device));
-      CK(cudaMemsetAsync(g->steal_counters + DRT_MULTI_MAX_CHUNKS + c, 0, sizeof(unsigned long long), g->stream));
-      if ((rc = barrier())) return rc;
-      for (int i = 0; i < n; i++) {
-        CK(cudaSetDevice(scenes[i]->device));
-        unsigned long long* cc = g->steal_counters + DRT_MULTI_MAX_CHUNKS + c;
-        rc = DRT_BY_PRECISION(plans[i], stageCloud<double>(scenes[i], plans[i], g->need, g->bg, cc), stageCloud<float>(scenes[i], plans[i], g->need, g->bg, cc));
-        if (rc) return rc;
-      }
-      if ((rc = barrier())) return rc;
-      for (int i = 1; i < n; i++) {
-        CK(cudaSetDevice(scenes[i]->device));
-        CK(cudaMemcpyAsync(scenes[i]->need, g->need, lp0.n_corners, cudaMemcpyDeviceToDevice, scenes[i]->stream));
-        CK(cudaMemcpyAsync(scenes[i]->bg, g->bg, lp0.n_corners * sizeof(float4), cudaMemcpyDeviceToDevice, scenes[i]->stream));
-      }
-    }
-    for (int i = 0; i < n; i++) {
-      CK(cudaSetDevice(scenes[i]->device));
-      int rc = DRT_BY_PRECISION(plans[i], stageResolve<double>(scenes[i], plans[i], c), stageResolve<float>(scenes[i], plans[i], c));
-      if (rc) return rc;
-    }
-    // the next chunk's marks and colours go into the gathering device's maps: its resolve must have read them first
-    if (lp0.perlin && c + 1 < lp0.n_chunks) { int rc = barrier(); if (rc) return rc; }
-  }
-  for (int i = 0; i < n; i++) {
-    CK(cudaSetDevice(scenes[i]->device));
-    int rc = stageEnd(scenes[i], plans[i], counters ? &counters[i] : nullptr);
-    if (rc) return rc;
-  }
+  int rc = st->precision == DRT_PRECISION_FP32 ? launchMulti<float>(scenes, n, *st, cam, *tile, pool_cap, counters, mc)
+                                               : launchMulti<double>(scenes, n, *st, cam, *tile, pool_cap, counters, mc);
+  if (rc) return rc;
   // the gathering stream waits for everyone's pixels, then one copy to the host
-  Counts hc[64]; int overflowed[64];
   for (int i = 1; i < n; i++) {
     CK(cudaSetDevice(scenes[i]->device));
     CK(cudaEventRecord(scenes[i]->ev_sync, scenes[i]->stream));
@@ -1096,22 +1046,12 @@ int renderMulti(drt_scene* const* scenes, int n, const drt_settings* st, const d
   CK(cudaSetDevice(g->device));
   for (int i = 1; i < n; i++) CK(cudaStreamWaitEvent(g->stream, scenes[i]->ev_sync, 0));
   CK(cudaMemcpyAsync(out_u8, g->out_u8, n_out, cudaMemcpyDeviceToHost, g->stream));
-  for (int i = 0; i < n; i++) {
-    drt_scene* s = scenes[i];
-    CK(cudaSetDevice(s->device));
-    memset(&hc[i], 0, sizeof(Counts)); overflowed[i] = 0;
-    if (counters && counters[i].collect) CK(cudaMemcpyAsync(&hc[i], s->counts, sizeof(Counts), cudaMemcpyDeviceToHost, s->stream));
-    CK(cudaMemcpyAsync(&overflowed[i], s->overflow, sizeof(int), cudaMemcpyDeviceToHost, s->stream));
-  }
-  int rc_all = DRT_OK;
   for (int i = n - 1; i >= 0; i--) {                            // the gathering stream (0) last: it waits for the others
-    drt_scene* s = scenes[i];
-    CK(cudaSetDevice(s->device));
-    CK(cudaStreamSynchronize(s->stream));
-    const int rc = finishRender(s, st, counters ? &counters[i] : nullptr, hc[i], overflowed[i]);
-    if (rc) rc_all = rc;
+    CK(cudaSetDevice(scenes[i]->device));
+    const int rc_i = readBack(scenes[i], counters ? &counters[i] : nullptr, true);
+    if (rc_i) rc = rc_i;
   }
-  return rc_all;
+  return rc;
 }
 
 }  // namespace
@@ -1190,8 +1130,8 @@ int drt_scene_create(const drt_scene_desc* d, int device, drt_scene** out) {
     dims.push_back(make_int2(t.width, t.height));
   }
   if (d->n_textures > 0) {
-    if (cudaMalloc(&s->d_tex, sizeof(cudaTextureObject_t) * d->n_textures) != cudaSuccess ||
-        cudaMalloc(&s->d_texdims, sizeof(int2) * d->n_textures) != cudaSuccess ||
+    if (s->d_tex.reserve(sizeof(cudaTextureObject_t) * d->n_textures) != cudaSuccess ||
+        s->d_texdims.reserve(sizeof(int2) * d->n_textures) != cudaSuccess ||
         cudaMemcpy(s->d_tex, s->tex_objs.data(), sizeof(cudaTextureObject_t) * d->n_textures, cudaMemcpyHostToDevice) != cudaSuccess ||
         cudaMemcpy(s->d_texdims, dims.data(), sizeof(int2) * d->n_textures, cudaMemcpyHostToDevice) != cudaSuccess)
       return bail(fail(DRT_ERR_CUDA, "texture table upload failed"));
@@ -1248,17 +1188,12 @@ void drt_scene_destroy(drt_scene* s) {
   if (s->stream) cudaStreamSynchronize(s->stream);
   for (auto t : s->tex_objs) cudaDestroyTextureObject(t);
   for (auto a : s->tex_arrays) cudaFreeArray(a);
-  void* ptrs[] = {s->dd.gbounds, s->df.gbounds, s->dd.geoms, s->dd.prims, s->dd.lights, s->dd.nodes, s->df.geoms, s->df.prims, s->df.lights, s->df.nodes, s->d_tex, s->d_texdims,
-                  s->samples, s->need, s->bg, s->out_u8, s->out_f32, s->counts, s->pool, s->batch_counter, s->overflow,
-                  s->steal_counters, s->owned};
-  for (void* p : ptrs) if (p) cudaFree(p);
-  freeMesh(&s->mesh);
   if (s->stage.base) cudaFreeHost(s->stage.base);
   if (s->ev0) cudaEventDestroy(s->ev0);
   if (s->ev1) cudaEventDestroy(s->ev1);
   if (s->ev_sync) cudaEventDestroy(s->ev_sync);
   if (s->stream) cudaStreamDestroy(s->stream);
-  delete s;
+  delete s;                       // frees the scene's device buffers (DevBuf)
 }
 
 // ---- mocap skeletons: parse + device forward kinematics live in drt_skeleton.cu ------------
@@ -1389,12 +1324,8 @@ void drt_abi_sizes(int32_t* out6) {
 // (drt_bvh_order.h): primitive indices, `cap` entries at most; returns the count.  Host only.
 int drt_debug_candidate_order(const drt_prim* prims, int32_t n_prims, int32_t* out, int32_t cap) {
   if (!prims || n_prims < 1 || !out) return 0;
-  std::vector<double> centers(3 * (size_t)n_prims);
-  for (int i = 0; i < n_prims; i++) for (int a = 0; a < 3; a++) centers[3 * i + a] = prims[i].center[a];
-  ReferenceBVH bvh;
-  bvh.build(centers.data(), n_prims, [&](int prim, double lo[3], double hi[3]) { primBounds(prims[prim], lo, hi); });
   int n = 0;
-  for (int i : bvh.order) { if (n < cap) out[n] = i; n++; }
+  for (int i : referenceBVH(prims, n_prims).order) { if (n < cap) out[n] = i; n++; }
   return n;
 }
 

@@ -21,6 +21,7 @@
 #include <stdint.h>
 #include <float.h>
 #include <math.h>
+#include <utility>
 
 #include "drt_rng.cuh"
 
@@ -199,12 +200,12 @@ struct Params {
   int x0, y0, w, h;
   // scene
   const Geom<R>* geoms; int n_geoms;
-  const float4* gbounds;    // slab-filter table: 3 float4 per PAIR of geoms (centre / half-extent, see slabMask)
-  const float4* geom_tree;  // 4-wide tree over the geoms (128-byte nodes as in drt_lbvh.cuh) for scenes beyond DRT_SMEM_GEOMS, or nullptr
+  const float4* gbounds;    // slab-filter table: one pair record per PAIR of geoms (drt_box.cuh, see slabMask)
+  const float4* geom_tree;  // 4-wide tree over the geoms (nodes of drt_box.cuh) for scenes beyond DRT_SMEM_GEOMS, or nullptr
   const NodeD<R>* nodes; int n_nodes;
   const PrimD<R>* prims;
   const LightD<R>* lights; int n_lights;
-  // triangle mesh (optional): LBVH nodes (4 float4 each), exact-test records, material = prims[mesh_prim]
+  // triangle mesh (optional): LBVH nodes (drt_box.cuh, 8 float4 each), exact-test records, material = prims[mesh_prim]
   const float4* mesh_nodes; const MeshTri<R>* mesh_tris; int n_mesh_tris; int mesh_prim;
   const unsigned short* mesh_mat;   // per-triangle material: prims[mesh_prim + mesh_mat[tri]]; nullptr: prims[mesh_prim]
   Vec<R> mesh_vel;                  // DRT_BLUR_VELOCITY: the mesh moves as a whole by mesh_vel * time (its materials' common velocity)
@@ -243,5 +244,28 @@ __host__ __device__ inline float clampf(float v) {  // helpers.h:230-235
   else if (v > 1.0f) return 1.0f;
   return v;
 }
+
+// Host side: device memory that frees itself.  Grow-only, move-only; reads as a T* wherever one is expected.
+template <typename T>
+struct DevBuf {
+  T* p = nullptr;
+  size_t cap = 0;   // bytes
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  DevBuf(DevBuf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+  DevBuf& operator=(DevBuf&& o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); return *this; }
+  ~DevBuf() { if (p) cudaFree(p); }
+  // at least `bytes`; a buffer that is already large enough is kept, a smaller one is replaced (contents lost)
+  cudaError_t reserve(size_t bytes) {
+    if (bytes <= cap) return cudaSuccess;
+    if (p) cudaFree(p);
+    p = nullptr; cap = 0;
+    const cudaError_t e = cudaMalloc(&p, bytes);
+    if (e == cudaSuccess) cap = bytes; else p = nullptr;
+    return e;
+  }
+  operator T*() const { return p; }
+};
 
 }  // namespace drt

@@ -8,19 +8,13 @@
 // collapse into 4-WIDE nodes: every binary node at even depth becomes a traversal node whose children are its
 // grandchildren (or a child that is a leaf), so a ray takes half as many dependent node fetches.
 //
-// Traversal node (float4 x 8 = 128 B, one cache line), children boxes as CENTRE / HALF-EXTENT in the pair-record layout
-// of the analytic slab filter (drt_kernels.cuh: slabPair), so both levels share the packed FFMA2 test:
-//   [0..2] {cx0 cx1 cy0 cy1} {cz0 cz1 hx0 hx1} {hy0 hy1 hz0 hz1}   children 0, 1
-//   [3..5] the same for children 2, 3
-//   [6]    child references as int bits: >= 0 traversal node index; < 0 leaf, triangle id = -ref - 1
-//   [7]    padding
-// An empty slot (children 2 and 3 only) has half-extent -1e30 and the reference 0x80000000: it never passes, not even for
-// an axis-parallel ray whose slab terms are NaN.
+// Traversal node: the 4-wide node of drt_box.cuh, so the LBVH and the slab filter share the packed FFMA2 test.
 #pragma once
 #include <cuda_runtime.h>
 #include <cub/device/device_radix_sort.cuh>
 #include <stdint.h>
 
+#include "drt_box.cuh"
 #include "drt_device.cuh"
 
 namespace drt {
@@ -127,13 +121,6 @@ __global__ void lbvh_refit(int n, const int* __restrict__ ids, const float4* __r
   }
 }
 
-// centre / half-extent of [lo, hi], rounded so that [c - h, c + h] contains it
-__device__ __forceinline__ void lbvh_centre_half(const float lo, const float hi, float& c, float& h) {
-  c = (float)(0.5 * ((double)lo + (double)hi));
-  const double hd = fmax((double)hi - (double)c, (double)c - (double)lo);
-  h = nextafterf(__double2float_ru(hd), INFINITY);
-}
-
 // collapse into the 128-byte 4-wide traversal nodes: one thread per binary internal node, even depths only
 __global__ void lbvh_pack4(int n, const int* __restrict__ ids, const float4* __restrict__ tlo, const float4* __restrict__ thi,
                            const int* __restrict__ left, const int* __restrict__ right, const int* __restrict__ parent_internal,
@@ -151,25 +138,15 @@ __global__ void lbvh_pack4(int n, const int* __restrict__ ids, const float4* __r
   }
   float cc[4][3], hh[4][3]; int ref[4];
   for (int k = 0; k < 4; k++) {
-    ref[k] = (int)0x80000000;
-    for (int a = 0; a < 3; a++) { cc[k][a] = 0.f; hh[k][a] = -1e30f; }
     if (k >= m) continue;
     float4 lo, hi;
     if (c[k] >= 0) { lo = nlo[c[k]]; hi = nhi[c[k]]; ref[k] = c[k]; }
     else { const int t = ids[-c[k] - 1]; lo = tlo[t]; hi = thi[t]; ref[k] = -(t + 1); }
-    lbvh_centre_half(lo.x, hi.x, cc[k][0], hh[k][0]);
-    lbvh_centre_half(lo.y, hi.y, cc[k][1], hh[k][1]);
-    lbvh_centre_half(lo.z, hi.z, cc[k][2], hh[k][2]);
+    centreHalf(lo.x, hi.x, cc[k][0], hh[k][0]);
+    centreHalf(lo.y, hi.y, cc[k][1], hh[k][1]);
+    centreHalf(lo.z, hi.z, cc[k][2], hh[k][2]);
   }
-  float4* nd = nodes + 8 * (size_t)i;
-  for (int p = 0; p < 2; p++) {
-    const int a = 2 * p, b = 2 * p + 1;
-    nd[3 * p + 0] = make_float4(cc[a][0], cc[b][0], cc[a][1], cc[b][1]);
-    nd[3 * p + 1] = make_float4(cc[a][2], cc[b][2], hh[a][0], hh[b][0]);
-    nd[3 * p + 2] = make_float4(hh[a][1], hh[b][1], hh[a][2], hh[b][2]);
-  }
-  nd[6] = make_float4(__int_as_float(ref[0]), __int_as_float(ref[1]), __int_as_float(ref[2]), __int_as_float(ref[3]));
-  nd[7] = make_float4(0.f, 0.f, 0.f, 0.f);
+  packNode4(nodes + 8 * (size_t)i, m, cc, hh, ref);
 }
 
 // exact-test records: the three vertices in the vector scalar R (the reference recomputes B-A,

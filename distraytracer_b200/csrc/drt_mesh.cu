@@ -3,6 +3,7 @@
 #include <cmath>
 #include <vector>
 
+#include "drt_box.cuh"
 #include "drt_lbvh.cuh"
 #include "drt_mesh.h"
 
@@ -11,17 +12,8 @@ namespace drt {
 #define MCK(call)                                                                           \
   do {                                                                                      \
     cudaError_t e_ = (call);                                                                \
-    if (e_ != cudaSuccess) { err = std::string(#call) + " failed: " + cudaGetErrorString(e_); goto fail; } \
+    if (e_ != cudaSuccess) { err = std::string(#call) + " failed: " + cudaGetErrorString(e_); return DRT_ERR_CUDA; } \
   } while (0)
-
-void freeMesh(MeshBuffers* m) {
-  if (!m) return;
-  if (m->nodes) cudaFree(m->nodes);
-  if (m->tris_f64) cudaFree(m->tris_f64);
-  if (m->tris_f32) cudaFree(m->tris_f32);
-  if (m->mat_ids) cudaFree(m->mat_ids);
-  *m = MeshBuffers();
-}
 
 int buildMesh(const drt_mesh* mesh, MeshBuffers* out, std::string& err) {
   const long long nv = mesh->n_vertices, nt = mesh->n_triangles;
@@ -43,96 +35,69 @@ int buildMesh(const drt_mesh* mesh, MeshBuffers* out, std::string& err) {
   float3 slo = make_float3(lo[0], lo[1], lo[2]);
   const float sinv = 1.0f / std::max(std::max(hi[0] - lo[0], hi[1] - lo[1]), std::max(hi[2] - lo[2], 1e-20f));   // cubic Morton cells
 
-  float *d_verts = nullptr, *d_tc = nullptr; int* d_idx = nullptr;
-  float4 *tlo = nullptr, *thi = nullptr, *nlo = nullptr, *nhi = nullptr;
-  uint64_t *codes = nullptr, *codes2 = nullptr; int *ids = nullptr, *ids2 = nullptr;
-  int *left = nullptr, *right = nullptr, *pin = nullptr, *pleaf = nullptr, *visits = nullptr;
-  void* tmp = nullptr; size_t tmp_bytes = 0;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  DevBuf<float> d_verts, d_tc; DevBuf<int> d_idx;
+  DevBuf<float4> tlo, thi, nlo, nhi;
+  DevBuf<uint64_t> codes, codes2; DevBuf<int> ids, ids2;
+  DevBuf<int> left, right, pin, pleaf, visits;
+  DevBuf<char> tmp; size_t tmp_bytes = 0;
   MeshBuffers mb;
   mb.n_tris = n;
   const int B = 256, G = (n + B - 1) / B;
-  MCK(cudaMalloc(&d_verts, sizeof(float) * 3 * nv));
-  MCK(cudaMalloc(&d_idx, sizeof(int) * 3 * nt));
+  MCK(d_verts.reserve(sizeof(float) * 3 * nv));
+  MCK(d_idx.reserve(sizeof(int) * 3 * nt));
   MCK(cudaMemcpy(d_verts, mesh->vertices, sizeof(float) * 3 * nv, cudaMemcpyHostToDevice));
   MCK(cudaMemcpy(d_idx, mesh->indices, sizeof(int) * 3 * nt, cudaMemcpyHostToDevice));
   if (mesh->texcoords) {
-    MCK(cudaMalloc(&d_tc, sizeof(float) * 2 * nv));
+    MCK(d_tc.reserve(sizeof(float) * 2 * nv));
     MCK(cudaMemcpy(d_tc, mesh->texcoords, sizeof(float) * 2 * nv, cudaMemcpyHostToDevice));
   }
-  MCK(cudaMalloc(&tlo, sizeof(float4) * n)); MCK(cudaMalloc(&thi, sizeof(float4) * n));
-  MCK(cudaMalloc(&nlo, sizeof(float4) * std::max(1, n - 1))); MCK(cudaMalloc(&nhi, sizeof(float4) * std::max(1, n - 1)));
-  MCK(cudaMalloc(&codes, sizeof(uint64_t) * n)); MCK(cudaMalloc(&codes2, sizeof(uint64_t) * n));
-  MCK(cudaMalloc(&ids, sizeof(int) * n)); MCK(cudaMalloc(&ids2, sizeof(int) * n));
-  MCK(cudaMalloc(&left, sizeof(int) * std::max(1, n - 1))); MCK(cudaMalloc(&right, sizeof(int) * std::max(1, n - 1)));
-  MCK(cudaMalloc(&pin, sizeof(int) * std::max(1, n - 1))); MCK(cudaMalloc(&pleaf, sizeof(int) * n));
-  MCK(cudaMalloc(&visits, sizeof(int) * std::max(1, n - 1)));
-  MCK(cudaMalloc(&mb.nodes, sizeof(float4) * 8 * std::max(1, n - 1)));
-  MCK(cudaMalloc(&mb.tris_f64, sizeof(MeshTri<double>) * n));
-  MCK(cudaMalloc(&mb.tris_f32, sizeof(MeshTri<float>) * n));
+  MCK(tlo.reserve(sizeof(float4) * n)); MCK(thi.reserve(sizeof(float4) * n));
+  MCK(nlo.reserve(sizeof(float4) * std::max(1, n - 1))); MCK(nhi.reserve(sizeof(float4) * std::max(1, n - 1)));
+  MCK(codes.reserve(sizeof(uint64_t) * n)); MCK(codes2.reserve(sizeof(uint64_t) * n));
+  MCK(ids.reserve(sizeof(int) * n)); MCK(ids2.reserve(sizeof(int) * n));
+  MCK(left.reserve(sizeof(int) * std::max(1, n - 1))); MCK(right.reserve(sizeof(int) * std::max(1, n - 1)));
+  MCK(pin.reserve(sizeof(int) * std::max(1, n - 1))); MCK(pleaf.reserve(sizeof(int) * n));
+  MCK(visits.reserve(sizeof(int) * std::max(1, n - 1)));
+  MCK(mb.nodes.reserve(sizeof(float4) * 8 * std::max(1, n - 1)));
+  MCK(mb.tris_f64.reserve(sizeof(MeshTri<double>) * n));
+  MCK(mb.tris_f32.reserve(sizeof(MeshTri<float>) * n));
   if (mesh->n_materials > 0) {
     std::vector<unsigned short> ids((size_t)n);
     for (int t = 0; t < n; t++) ids[t] = (unsigned short)mesh->material_ids[t];
-    MCK(cudaMalloc(&mb.mat_ids, sizeof(unsigned short) * n));
+    MCK(mb.mat_ids.reserve(sizeof(unsigned short) * n));
     MCK(cudaMemcpy(mb.mat_ids, ids.data(), sizeof(unsigned short) * n, cudaMemcpyHostToDevice));
   }
-  MCK(cudaEventCreate(&e0)); MCK(cudaEventCreate(&e1));
-  MCK(cudaEventRecord(e0));
   lbvh_tri_setup<<<G, B>>>(n, d_verts, d_idx, slo, sinv, tlo, thi, codes, ids);
-  lbvh_tri_records<double><<<G, B>>>(n, d_verts, d_idx, d_tc, (MeshTri<double>*)mb.tris_f64);
-  lbvh_tri_records<float><<<G, B>>>(n, d_verts, d_idx, d_tc, (MeshTri<float>*)mb.tris_f32);
+  lbvh_tri_records<double><<<G, B>>>(n, d_verts, d_idx, d_tc, mb.tris_f64);
+  lbvh_tri_records<float><<<G, B>>>(n, d_verts, d_idx, d_tc, mb.tris_f32);
   if (n > 1) {
-    MCK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, codes, codes2, ids, ids2, n, 0, 63));
-    MCK(cudaMalloc(&tmp, tmp_bytes));
-    MCK(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, codes, codes2, ids, ids2, n, 0, 63));
+    MCK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, codes.p, codes2.p, ids.p, ids2.p, n, 0, 63));
+    MCK(tmp.reserve(tmp_bytes));
+    MCK(cub::DeviceRadixSort::SortPairs(tmp.p, tmp_bytes, codes.p, codes2.p, ids.p, ids2.p, n, 0, 63));
     MCK(cudaMemset(visits, 0, sizeof(int) * (n - 1)));
     lbvh_karras<<<(n - 1 + B - 1) / B, B>>>(n, codes2, left, right, pin, pleaf);
     lbvh_refit<<<G, B>>>(n, ids2, tlo, thi, left, right, pin, pleaf, nlo, nhi, visits);
     lbvh_pack4<<<(n - 1 + B - 1) / B, B>>>(n, ids2, tlo, thi, left, right, pin, nlo, nhi, mb.nodes);
   } else {
-    // single triangle: one node
+    // single triangle: one node whose slots 0 and 1 both hold it (only slots 2 and 3 may be empty); a second test of it
+    // changes nothing
     float4 h_lo, h_hi;
     MCK(cudaMemcpy(&h_lo, tlo, sizeof(float4), cudaMemcpyDeviceToHost));
     MCK(cudaMemcpy(&h_hi, thi, sizeof(float4), cudaMemcpyDeviceToHost));
-    float c[3], h[3];
-    const float l3[3] = {h_lo.x, h_lo.y, h_lo.z}, u3[3] = {h_hi.x, h_hi.y, h_hi.z};
+    float c[4][3], h[4][3];
+    int ref[4] = {-1, -1};
     for (int a = 0; a < 3; a++) {
-      c[a] = (float)(0.5 * ((double)l3[a] + (double)u3[a]));
-      const double hd = std::max((double)u3[a] - (double)c[a], (double)c[a] - (double)l3[a]);
-      float hf = (float)hd;
-      if ((double)hf < hd) hf = nextafterf(hf, INFINITY);
-      h[a] = nextafterf(hf, INFINITY);
+      centreHalf((&h_lo.x)[a], (&h_hi.x)[a], c[0][a], h[0][a]);
+      c[1][a] = c[0][a]; h[1][a] = h[0][a];
     }
-    const float E = -1e30f;
-    const int leaf = -1, none = (int)0x80000000;
     float4 nd[8];
-    // slots 0 and 1 both hold the triangle (only slots 2 and 3 may be empty); a second test of it changes nothing
-    nd[0] = make_float4(c[0], c[0], c[1], c[1]); nd[1] = make_float4(c[2], c[2], h[0], h[0]); nd[2] = make_float4(h[1], h[1], h[2], h[2]);
-    nd[3] = make_float4(0.f, 0.f, 0.f, 0.f); nd[4] = make_float4(0.f, 0.f, E, E); nd[5] = make_float4(E, E, E, E);
-    memcpy(&nd[6].x, &leaf, 4); memcpy(&nd[6].y, &leaf, 4); memcpy(&nd[6].z, &none, 4); memcpy(&nd[6].w, &none, 4);
-    nd[7] = make_float4(0.f, 0.f, 0.f, 0.f);
+    packNode4(nd, 2, c, h, ref);
     MCK(cudaMemcpy(mb.nodes, nd, sizeof(nd), cudaMemcpyHostToDevice));
   }
-  MCK(cudaEventRecord(e1));
   MCK(cudaDeviceSynchronize());
   MCK(cudaGetLastError());
-  cudaEventElapsedTime(&mb.build_ms, e0, e1);
-  *out = mb;
-  {
-    void* frees[] = {d_verts, d_tc, d_idx, tlo, thi, nlo, nhi, codes, codes2, ids, ids2, left, right, pin, pleaf, visits, tmp};
-    for (void* p : frees) if (p) cudaFree(p);
-    cudaEventDestroy(e0); cudaEventDestroy(e1);
-  }
+  *out = std::move(mb);
   return DRT_OK;
-fail:
-  {
-    void* frees[] = {d_verts, d_tc, d_idx, tlo, thi, nlo, nhi, codes, codes2, ids, ids2, left, right, pin, pleaf, visits, tmp};
-    for (void* p : frees) if (p) cudaFree(p);
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-    freeMesh(&mb);
-  }
-  return DRT_ERR_CUDA;
 }
 
 }  // namespace drt

@@ -3,17 +3,16 @@
 #include <string>
 #include <cuda_runtime.h>
 #include "../../include/drt.h"
+#include "drt_device.cuh"
 
 namespace drt {
 struct MeshBuffers {
-  float4* nodes = nullptr;   // 4 float4 per internal node
-  void* tris_f64 = nullptr;  // MeshTri<double>[n_tris]
-  void* tris_f32 = nullptr;  // MeshTri<float>[n_tris]
-  unsigned short* mat_ids = nullptr;  // per-triangle index into the mesh's material table, or nullptr (one material)
+  DevBuf<float4> nodes;              // 4-wide LBVH nodes (drt_box.cuh), 8 float4 per node
+  DevBuf<MeshTri<double>> tris_f64;  // [n_tris]
+  DevBuf<MeshTri<float>> tris_f32;   // [n_tris]
+  DevBuf<unsigned short> mat_ids;    // per-triangle index into the mesh's material table, or empty (one material)
   int n_tris = 0;
-  float build_ms = 0;        // device time of the build (CUDA events)
 };
 // Uploads the mesh, builds the LBVH on the current device.  Returns a drt_status.
 int buildMesh(const drt_mesh* mesh, MeshBuffers* out, std::string& err);
-void freeMesh(MeshBuffers* m);
 }  // namespace drt
