@@ -653,7 +653,10 @@ void fillParams(Params<R>& P, const drt_scene* s, const DevScene<R>& ds, const d
   f3(P.bluesky, st.bluesky); f3(P.redsky, st.redsky);
   P.saturation = st.saturation; P.clouddist = st.clouddist; P.cloudhoff = st.cloudhoff;
   P.x0 = tile.x0; P.y0 = tile.y0; P.w = tile.width; P.h = tile.height;
-  P.geoms = ds.geoms; P.n_geoms = ds.n_geoms; P.gbounds = ds.gbounds; P.geom_tree = ds.geom_tree >= 0 ? ds.gbounds + ds.geom_tree : nullptr; P.nodes = ds.nodes; P.n_nodes = ds.n_nodes; P.prims = ds.prims; P.lights = ds.lights; P.n_lights = ds.n_lights;
+  P.geoms = ds.geoms; P.n_geoms = ds.n_geoms; P.gbounds = ds.gbounds; P.geom_tree = ds.geom_tree >= 0 ? ds.gbounds + ds.geom_tree : nullptr; P.nodes = ds.nodes; P.n_nodes = ds.n_nodes; P.prims = ds.prims; P.n_prims = ds.n_prims; P.lights = ds.lights; P.n_lights = ds.n_lights;
+  // render_wave serves the records from shared memory when they fit; big scenes (FT_BIG) keep them in global memory
+  const size_t recs = sizeof(Geom<R>) * ds.n_geoms + sizeof(PrimD<R>) * ds.n_prims + sizeof(LightD<R>) * ds.n_lights;
+  P.smem_recs = (ds.n_geoms <= DRT_SMEM_GEOMS && recs <= DRT_SMEM_RECS) ? (int)recs : 0;
   P.tex = s->d_tex; P.texdims = s->d_texdims;
   if (s->has_mesh) {
     P.mesh_nodes = s->mesh.nodes; P.n_mesh_tris = s->mesh.n_tris; P.mesh_prim = (int)s->prims.size();

@@ -14,7 +14,8 @@
 //              candidates is what RectPrismV2::intersect computes (815-838).
 //   PrimD<R> : the per-GeoPrimitive shading record (material, normal, UV, emissive).
 //   LightD<R>: the LightPrimitive records.
-// Records are 16-byte aligned; every lane of a warp reads the same record in the
+// Records are 16-byte aligned and whole 16-byte words (render_wave copies them to shared
+// memory word by word); every lane of a warp reads the same record in the
 // candidate loops, so loads are warp-uniform broadcasts.
 #pragma once
 #include <cuda_runtime.h>
@@ -203,8 +204,9 @@ struct Params {
   const float4* gbounds;    // slab-filter table: one pair record per PAIR of geoms (drt_box.cuh, see slabMask)
   const float4* geom_tree;  // 4-wide tree over the geoms (nodes of drt_box.cuh) for scenes beyond DRT_SMEM_GEOMS, or nullptr
   const NodeD<R>* nodes; int n_nodes;
-  const PrimD<R>* prims;
+  const PrimD<R>* prims; int n_prims;
   const LightD<R>* lights; int n_lights;
+  int smem_recs;            // bytes of geoms + prims + lights when they fit DRT_SMEM_RECS (an FT_RECS render_wave stages them), else 0
   // triangle mesh (optional): LBVH nodes (drt_box.cuh, 8 float4 each), exact-test records, material = prims[mesh_prim]
   const float4* mesh_nodes; const MeshTri<R>* mesh_tris; int n_mesh_tris; int mesh_prim;
   const unsigned short* mesh_mat;   // per-triangle material: prims[mesh_prim + mesh_mat[tri]]; nullptr: prims[mesh_prim]

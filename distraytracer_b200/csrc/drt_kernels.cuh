@@ -417,6 +417,31 @@ struct HitRec {
   int checker_sel;  // 0: keep prim colour, 1: color1, 2: color2
 };
 
+// render_wave's dynamic shared memory: [ acc: slots x 3 x u64 | flags: slots x u32 | order: hits x u16 | hkey: hits x u8 ]
+// (waveDynSmemBytes), then, in FT_RECS instantiations, the scene records [ geoms | prims | lights ] (Params::smem_recs)
+extern __shared__ __align__(16) unsigned char s_dyn[];
+__host__ __device__ constexpr size_t waveDynSmemBytes() { return (size_t)DRT_CTA_SLOTS * 28 + (size_t)DRT_CTA_HITS * 3; }
+static_assert(waveDynSmemBytes() % 16 == 0, "the staged records start on a 16-byte boundary");
+
+// The geom, primitive and light tables: the CTA's copy in shared memory in FT_RECS instantiations (every exact test and
+// every shading step starts with loads from them; from global memory half of them missed the L1), else the global tables.
+template <typename R, int F>
+__device__ __forceinline__ const Geom<R>* geomRecs(const Params<R>& P) {
+  return (F & FT_RECS) ? (const Geom<R>*)(s_dyn + waveDynSmemBytes()) : P.geoms;
+}
+template <typename R, int F>
+__device__ __forceinline__ const PrimD<R>* primRecs(const Params<R>& P) {
+  return (F & FT_RECS) ? (const PrimD<R>*)(geomRecs<R, F>(P) + P.n_geoms) : P.prims;
+}
+template <typename R, int F>
+__device__ __forceinline__ const LightD<R>* lightRecs(const Params<R>& P) {
+  return (F & FT_RECS) ? (const LightD<R>*)(primRecs<R, F>(P) + P.n_prims) : P.lights;
+}
+// render_wave's staging copy, by the whole CTA; the records are alignas(16), so whole 16-byte words
+__device__ __forceinline__ void ctaCopy16(void* dst, const void* src, const int bytes) {
+  for (int i = threadIdx.x; i < bytes / 16; i += blockDim.x) ((uint4*)dst)[i] = __ldg((const uint4*)src + i);
+}
+
 // One candidate of the closest-hit search: the intersect() of the geom's class.
 template <typename R, int F>
 __device__ inline bool geomIntersect(const Params<R>& P, const Geom<R>& g, int gi, const int type, const Moved<R>& mv,
@@ -424,7 +449,7 @@ __device__ inline bool geomIntersect(const Params<R>& P, const Geom<R>& g, int g
   bool ok = false;
   inside = 0; sel = 0;
     if ((F & FT_BOX) && type == G_BOX) {
-      return boxIntersect<R>(P.prims[g.owner], shiftPoint<R, F>(mv, 0, g.vel, g.p0), shiftPoint<R, F>(mv, 0, g.vel, g.p1), ray, start, t_hit, inside, sel);
+      return boxIntersect<R>(primRecs<R, F>(P)[g.owner], shiftPoint<R, F>(mv, 0, g.vel, g.p0), shiftPoint<R, F>(mv, 0, g.vel, g.p1), ray, start, t_hit, inside, sel);
     } else if (type == G_RECT || type == G_CHECKER) {
       Vec<R> A = shiftPoint<R, F>(mv, g.flags, g.vel, g.p0);
       if (type == G_CHECKER) {  // exact-zero edge path pinned to "no hit" (quirk Q17)
@@ -434,7 +459,7 @@ __device__ inline bool geomIntersect(const Params<R>& P, const Geom<R>& g, int g
       ok = rectHit<R>(A, g.p1, g.p2, g.p3, g.len1, g.len2, g.eps, ray, start, t_hit, c1, c2);
       if (ok && type == G_CHECKER) {
         if (g.flags & GF_HAS_HOLE) {  // CheckerboardWithHole: inner Rectangle cancels the hit (geometry.cpp:2408-2414)
-          const Geom<R>& hgeo = P.geoms[gi + 1];
+          const Geom<R>& hgeo = geomRecs<R, F>(P)[gi + 1];
           float th, d1, d2;
           if (rectHit<R>(hgeo.p0, hgeo.p1, hgeo.p2, hgeo.p3, hgeo.len1, hgeo.len2, hgeo.eps, ray, start, th, d1, d2))
             ok = false;
@@ -725,7 +750,7 @@ __device__ inline void closestHit(const Params<R>& P, const SlabTab gb, const Mo
         while (cur >= 0) { if (COUNT) cnt.node_tests += 4; cur = bvh4Visit<true>(P.geom_tree, cur, st, stack, sp, P.overflow); }
         if (cur == DRT_MESH_DONE) break;
         const int gi = -cur - 1;
-        const Geom<R>& g = P.geoms[gi];
+        const Geom<R>& g = geomRecs<R, F>(P)[gi];
         const int type = g.type;
         if (COUNT) cnt.geom_tests[type]++;
         float t_hit; int inside, sel;
@@ -746,7 +771,7 @@ __device__ inline void closestHit(const Params<R>& P, const SlabTab gb, const Mo
       while (mask) {
         const int gi = g0 + __ffs(mask) - 1;      // ascending = the reference's candidate order
         mask &= mask - 1;
-        const Geom<R>& g = P.geoms[gi];
+        const Geom<R>& g = geomRecs<R, F>(P)[gi];
         const int type = g.type;
         if (type == G_HOLE) continue;
         // a box whose entry lies beyond the best hit cannot hold a closer (or tying) one
@@ -773,7 +798,7 @@ __device__ inline void closestHit(const Params<R>& P, const SlabTab gb, const Mo
     if (!nd.leaf) { stack[sp++] = nd.left; stack[sp++] = nd.right; continue; }   // right child is popped first (:497-509)
     const int g_end = nd.first + nd.count;
     for (int gi = nd.first; gi < g_end; gi++) {
-      const Geom<R>& g = P.geoms[gi];
+      const Geom<R>& g = geomRecs<R, F>(P)[gi];
       const int type = g.type;
       if (type == G_HOLE) continue;
       if (COUNT) cnt.geom_tests[type]++;
@@ -793,7 +818,7 @@ __device__ inline bool geomShadow(const Params<R>& P, const Geom<R>& g, int gi, 
     t_occ = 0.0f;   // on success: a ray parameter at which the ray certainly touches the geom
     if ((F & FT_BOX) && type == G_BOX) {
       // t_occ stays 0: these classes report occlusion without a touch point, so the reference gather is always replayed
-      return boxShadow<R>(P.prims[g.owner], shiftPoint<R, F>(mv, 0, g.vel, g.p0), shiftPoint<R, F>(mv, 0, g.vel, g.p1), ray, start, t_max, aborted);
+      return boxShadow<R>(primRecs<R, F>(P)[g.owner], shiftPoint<R, F>(mv, 0, g.vel, g.p0), shiftPoint<R, F>(mv, 0, g.vel, g.p1), ray, start, t_max, aborted);
     } else if (type == G_RECT || type == G_CHECKER) {
       Vec<R> A = shiftPoint<R, F>(mv, g.flags, g.vel, g.p0);
       // Checkerboard inherits Rectangle::intersectShadow (eps 1e-4); CheckerboardWithHole
@@ -802,7 +827,7 @@ __device__ inline bool geomShadow(const Params<R>& P, const Geom<R>& g, int gi, 
       float th, c1, c2;
       if (rectHit<R>(A, g.p1, g.p2, g.p3, g.len1, g.len2, eps, ray, start, th, c1, c2) && th < t_max) {
         if (g.flags & GF_HAS_HOLE) {
-          const Geom<R>& hgeo = P.geoms[gi + 1];
+          const Geom<R>& hgeo = geomRecs<R, F>(P)[gi + 1];
           float t2, d1, d2;
           if (rectHit<R>(hgeo.p0, hgeo.p1, hgeo.p2, hgeo.p3, hgeo.len1, hgeo.len2, hgeo.eps, ray, start, t2, d1, d2) &&
               t2 < t_max)
@@ -891,7 +916,7 @@ __device__ inline bool anyHit(const Params<R>& P, const SlabTab gb, const Moved<
     const SlabRay sr = slabRay(ix, iy, iz, ox, oy, oz, t_max * 1.0001f + 1e-4f);
     // one candidate: 1 = the ray is occluded, -1 = the reference throws (slab-box prisms), 0 = go on
     auto candidate = [&](const int gi) -> int {
-      const Geom<R>& g = P.geoms[gi];
+      const Geom<R>& g = geomRecs<R, F>(P)[gi];
       const int type = g.type;
       if (type == G_HOLE || g.owner == skip_owner) return 0;     // an area light never shadows itself (832-837)
       if (COUNT) cnt.geom_tests[type]++;
@@ -943,7 +968,7 @@ __device__ inline bool anyHit(const Params<R>& P, const SlabTab gb, const Moved<
     if (!nd.leaf) { stack[sp++] = nd.left; stack[sp++] = nd.right; continue; }
     const int g_end = nd.first + nd.count;
     for (int gi = nd.first; gi < g_end; gi++) {
-      const Geom<R>& g = P.geoms[gi];
+      const Geom<R>& g = geomRecs<R, F>(P)[gi];
       const int type = g.type;
       if (type == G_HOLE) continue;
       if (g.owner == skip_owner) continue;
@@ -1183,8 +1208,8 @@ __device__ inline bool traceRay(const Params<R>& P, const SlabTab gb, const Task
   if ((F & (FT_VEL | FT_REFBLUR)) && (T.bits & TASK_CHAIN)) motion = 0;             // :519
   if (h.geom < 0) return false;                                         // :541-544
   if ((F & (FT_VEL | FT_REFBLUR)) && (T.bits & TASK_CHAIN)) {
-    const int owner = h.geom >= P.n_geoms ? meshOwner(P, h.geom - P.n_geoms) : P.geoms[h.geom].owner;
-    motion = (P.prims[owner].flags & 2) ? 1 : 0;                        // DRT_FLAG_MOTION, :564
+    const int owner = h.geom >= P.n_geoms ? meshOwner(P, h.geom - P.n_geoms) : geomRecs<R, F>(P)[h.geom].owner;
+    motion = (primRecs<R, F>(P)[owner].flags & 2) ? 1 : 0;                        // DRT_FLAG_MOTION, :564
   }
   return true;
 }
@@ -1247,8 +1272,8 @@ __device__ void shadeA(const Params<R>& P, const Task<R>& T, const HitRec& h, Ta
     const Vec<R> ray = T.dir, eye = T.org;
     const float k = T.k;
     const int mesh_tri = ((F & FT_MESH) && h.geom >= P.n_geoms) ? h.geom - P.n_geoms : -1;
-    const int owner = mesh_tri >= 0 ? meshOwner(P, mesh_tri) : P.geoms[h.geom].owner;
-    const PrimD<R>& pr = P.prims[owner];
+    const int owner = mesh_tri >= 0 ? meshOwner(P, mesh_tri) : geomRecs<R, F>(P)[h.geom].owner;
+    const PrimD<R>& pr = primRecs<R, F>(P)[owner];
 
     const Vec<R> isectP = eye + (R)h.t * ray;                           // :548
     // ---- getNorm of the hit class ------------------------------------------------
@@ -1436,7 +1461,7 @@ __device__ void shadeA(const Params<R>& P, const Task<R>& T, const HitRec& h, Ta
 template <typename R, int F, bool COUNT>
 __device__ void shadowPair(const Params<R>& P, const SlabTab gb, const PairIn<R>& in, int li, const PairOut<R>& out, const int oi,
                            Counts& cnt) {
-  const LightD<R>& L = P.lights[li];
+  const LightD<R>& L = lightRecs<R, F>(P)[li];
   const Vec<R> isectP = in.isectP;
   Moved<R> mv;                                      // makeMoved, with blurVal(P, dt) as shadeA evaluated it
   mv.val = (F & FT_REFBLUR) ? in.val : 0.0f;
@@ -1466,13 +1491,13 @@ __device__ void shadowPair(const Params<R>& P, const SlabTab gb, const PairIn<R>
 // The rest of the light loop (:856-959) for lights [l0, l1) of one hit, in order.
 template <typename R, int F, bool COUNT>
 __device__ void shadeB(const Params<R>& P, ShadeState<R>& S, const PairOut<R>& res, const int hit_lane, int l0, int l1, Counts& cnt) {
-  const PrimD<R>& pr = P.prims[S.prim];
+  const PrimD<R>& pr = primRecs<R, F>(P)[S.prim];
   for (int li = l0; li < l1 && !S.early && !S.aborted; li++) {
     const int oi = (li - l0) * 32 + hit_lane;                          // light-major: [light][hit]
     const int state = res.state[oi];
     if (state == 2) { S.aborted = true; break; }                     // throws geometry.cpp:2785-2789
     if (state == 0) continue;                                         // shadowed :852-855
-    const LightD<R>& L = P.lights[li];
+    const LightD<R>& L = lightRecs<R, F>(P)[li];
     Vec<R> sray;                                                      // as shadowPair drew it
     if (L.type == 0) sray = L.center - S.isectP;
     else if (L.type == 2) sray = rectSample<R>(L.A, L.B, L.D, S.path, rng_dim_light(li, 0)) - S.isectP;
@@ -1694,7 +1719,6 @@ __device__ __noinline__ void primaryRay(const Params<R>& P, long long gidx, cons
 #define DRT_WAVE_CTAS_PER_SM 1
 #endif
 #define DRT_HIT_BUCKETS 64     // hits are grouped by min(geom, 63) before SHADE
-__host__ __device__ constexpr size_t waveDynSmemBytes() { return (size_t)DRT_CTA_SLOTS * 28 + (size_t)DRT_CTA_HITS * 3; }
 template <typename R>
 __host__ __device__ constexpr size_t waveScratchBytes(int pool_cap) {
   return (size_t)pool_cap * sizeof(Task<R>) + DRT_CTA_HITS * sizeof(HitRef) + DRT_WAVE_WARPS * pairOutBytes<R>() +
@@ -1723,8 +1747,7 @@ __host__ __device__ constexpr size_t waveScratchBytes(int pool_cap) {
 // empty (depth 0, which TRACE skips like the reference's `depth == 0` return).
 template <typename R, int F, bool COUNT>
 __global__ void __launch_bounds__(32 * DRT_WAVE_WARPS, DRT_WAVE_CTAS_PER_SM) render_wave(const __grid_constant__ Params<R> P) {
-  // dynamic shared memory (waveDynSmemBytes): [ acc: slots x 3 x u64 | flags: slots x u32 | order: hits x u16 | hkey: hits x u8 ]
-  extern __shared__ __align__(16) unsigned char s_dyn[];
+  // dynamic shared memory: see s_dyn
   unsigned long long(*s_acc)[3] = (unsigned long long(*)[3])s_dyn;
   unsigned int* s_flags = (unsigned int*)(s_dyn + (size_t)DRT_CTA_SLOTS * 24);
   unsigned short* s_order = (unsigned short*)(s_dyn + (size_t)DRT_CTA_SLOTS * 28);
@@ -1740,6 +1763,11 @@ __global__ void __launch_bounds__(32 * DRT_WAVE_WARPS, DRT_WAVE_CTAS_PER_SM) ren
   if (!(F & FT_BIG) || P.n_geoms <= DRT_SMEM_GEOMS) {
     for (int i = threadIdx.x; i < slabPairWords(P.n_geoms) + 2 * ((P.n_geoms + 7) / 8); i += blockDim.x) s_gb[i] = P.gbounds[i];
     gb.s = (unsigned)__cvta_generic_to_shared(s_gb);
+  }
+  if (F & FT_RECS) {                  // the geom, primitive and light records (published by the barrier below)
+    ctaCopy16((void*)geomRecs<R, F>(P), P.geoms, P.n_geoms * (int)sizeof(Geom<R>));
+    ctaCopy16((void*)primRecs<R, F>(P), P.prims, P.n_prims * (int)sizeof(PrimD<R>));
+    ctaCopy16((void*)lightRecs<R, F>(P), P.lights, P.n_lights * (int)sizeof(LightD<R>));
   }
   const unsigned FULL = 0xffffffffu;
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, tid = threadIdx.x;

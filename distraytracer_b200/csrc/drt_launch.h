@@ -30,6 +30,10 @@
 #define DRT_PAIR_LIGHTS 8      // lights whose shadow rays are spread over the warp per pass
 #endif
 #define DRT_SMEM_GEOMS 256     // slab-filter entries staged in shared memory per CTA
+// Bytes of geom + primitive + light records staged in shared memory per CTA (FT_RECS); a scene with more reads them from
+// global memory.  With the CTA's other 65.0 KB of shared memory (11.3 KB static + 53.7 KB waveDynSmemBytes) and the 1 KB
+// reserved per block this stays within a 100 KB shared-memory carve-out: one CTA of 16 warps per SM, 156 KB of L1 left.
+#define DRT_SMEM_RECS (32 * 1024)
 
 // ---- feature mask of a render_wave instantiation ------------------------------------------------------------------
 // render_wave is compiled once per feature set and the host picks the smallest instantiation that covers the scene and
@@ -45,7 +49,12 @@ enum WaveFeat {
   FT_BIG = 32,      // more geoms than the shared-memory slab table holds (DRT_SMEM_GEOMS)
   FT_BOX = 64,      // slab-box prisms (RectPrism / RectPrismWithCylinder / RectPrismWithHoles) are present
   FT_SPILL = 128,   // a rectangle whose edges B-A, D-A are not orthogonal is present (GF_SPILL: hits need the reference's gather replayed)
-  FT_ALL = 255
+  FT_ALL = 255,
+  // Not a scene feature: the instantiation reads the geom, primitive and light records from a copy in shared memory, which
+  // the launcher picks when the scene's records fit (Params::smem_recs).  A compile-time choice: with the table picked at
+  // run time, the pointer select held registers and turned ld.shared into generic loads (the bench instantiation: 56-92
+  // bytes of spill stores instead of 20).  Every mask of DRT_WAVE_FEATS but FT_ALL is also instantiated with it.
+  FT_RECS = 256
 };
 
 // the instantiated masks (drt_launch_impl.cuh must hold one DRT_WAVE_CASE per entry); FT_ALL last
@@ -60,7 +69,8 @@ int waveFeatPick(int need);
 template <typename R> int waveGridBlocks();
 // bytes of scratch (ray pools of `pool_cap` tasks, hit buffers, shadow-pair buffers) a grid of `blocks` CTAs needs
 template <typename R> size_t wavePoolBytes(int blocks, int pool_cap);
-// `feat`: what the call needs (any mask; the launcher maps it to an instantiation).  Returns the mask launched.
+// `feat`: what the call needs (any mask; the launcher maps it to an instantiation, adding FT_RECS when P.smem_recs).
+// Returns the mask launched.
 template <typename R> int launchRenderSamples(const Params<R>& P, bool collect, int feat, int blocks, cudaStream_t q);
 // one translation unit per (precision, group) instantiates part of the list: kernel of mask `feat`, or nullptr
 template <typename R> using WaveFnT = void (*)(Params<R>);

@@ -7,7 +7,10 @@
 
 namespace drt {
 typedef WaveFnT<DRT_REAL> WaveFn;
-#define DRT_WAVE_CASE(mask) if (feat == (mask) && !collect) return render_wave<DRT_REAL, (mask), false>
+// each mask with and without FT_RECS (records in shared memory)
+#define DRT_WAVE_CASE(mask)                                                                                              \
+  if ((feat & ~FT_RECS) == (mask) && !collect)                                                                           \
+    return (feat & FT_RECS) ? render_wave<DRT_REAL, (mask) | FT_RECS, false> : render_wave<DRT_REAL, (mask), false>
 #if DRT_GROUP == 0
 // static scenes: the bench workload (glass + textures), plain and textured analytic scenes
 template <> WaveFn waveKernelOfGroup<DRT_REAL, 0>(int feat, bool collect) {
@@ -28,8 +31,7 @@ template <> WaveFn waveKernelOfGroup<DRT_REAL, 1>(int feat, bool collect) {
 // reference-mode motion blur, and the instantiation that can do everything (also the counting build)
 template <> WaveFn waveKernelOfGroup<DRT_REAL, 2>(int feat, bool collect) {
   DRT_WAVE_CASE(FT_REFBLUR | FT_GLASS | FT_TEX);
-  DRT_WAVE_CASE(FT_ALL);
-  if (feat == FT_ALL && collect) return render_wave<DRT_REAL, FT_ALL, true>;
+  if (feat == FT_ALL) return collect ? render_wave<DRT_REAL, FT_ALL, true> : render_wave<DRT_REAL, FT_ALL, false>;   // global records
   return nullptr;
 }
 #endif
@@ -46,20 +48,26 @@ template <> int waveGridBlocks<DRT_REAL>() {
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int* list = waveFeatList(&n);
-  for (int i = 0; i <= n; i++) {          // every instantiation + the counting build; the grid fits the hungriest one
-    WaveFn f = i < n ? waveKernel(list[i], false) : waveKernel(FT_ALL, true);
+  auto fit = [&](WaveFn f, const size_t smem) {
     int k = 0;
-    cudaFuncSetAttribute((const void*)f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)waveDynSmemBytes());
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&k, (const void*)f, 32 * DRT_WAVE_WARPS, waveDynSmemBytes());
+    cudaFuncSetAttribute((const void*)f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&k, (const void*)f, 32 * DRT_WAVE_WARPS, smem);
     per_sm = k < per_sm ? k : per_sm;
+  };
+  // every instantiation (FT_RECS: with a full record table) + the counting build; the grid fits the hungriest one
+  for (int i = 0; i < n; i++) {
+    fit(waveKernel(list[i], false), waveDynSmemBytes());
+    if (list[i] != FT_ALL) fit(waveKernel(list[i] | FT_RECS, false), waveDynSmemBytes() + DRT_SMEM_RECS);
   }
+  fit(waveKernel(FT_ALL, true), waveDynSmemBytes());
   if (per_sm < 1) per_sm = 1;
   return sms * per_sm;   // a whole multiple of the SM count: every SM holds the same number of persistent CTAs
 }
 template <> size_t wavePoolBytes<DRT_REAL>(int blocks, int pool_cap) { return (size_t)blocks * waveScratchBytes<DRT_REAL>(pool_cap); }
 template <> int launchRenderSamples<DRT_REAL>(const Params<DRT_REAL>& P, bool collect, int feat, int blocks, cudaStream_t q) {
-  const int pick = collect ? FT_ALL : waveFeatPick(feat);
-  waveKernel(pick, collect)<<<blocks, 32 * DRT_WAVE_WARPS, waveDynSmemBytes(), q>>>(P);
+  int pick = collect ? FT_ALL : waveFeatPick(feat);
+  if (pick != FT_ALL && P.smem_recs) pick |= FT_RECS;
+  waveKernel(pick, collect)<<<blocks, 32 * DRT_WAVE_WARPS, waveDynSmemBytes() + ((pick & FT_RECS) ? P.smem_recs : 0), q>>>(P);
   return pick;
 }
 template <> void launchCloudCorners<DRT_REAL>(const Params<DRT_REAL>& P, cudaStream_t q) {
