@@ -49,20 +49,16 @@ RectD makeRect(const D3& A, const D3& B, const D3& C, const D3& D) {
   return r;
 }
 
-// padded single-precision bounds for the slab filter (drt_kernels.cuh slabMayHit)
+// padded single-precision bounds for the slab filter (drt_kernels.cuh slabMayHit); `planar`: see padBounds in drt_box.cuh
 template <typename R>
-void setBounds(Geom<R>& g, const D3* pts, int n, double extra) {
+void setBounds(Geom<R>& g, const D3* pts, int n, double extra, bool planar) {
   double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
   for (int i = 0; i < n; i++) {
     const double v[3] = {pts[i].x, pts[i].y, pts[i].z};
     for (int a = 0; a < 3; a++) { lo[a] = std::min(lo[a], v[a] - extra); hi[a] = std::max(hi[a], v[a] + extra); }
   }
   float fl[3], fh[3];
-  for (int a = 0; a < 3; a++) {
-    const double pad = 1e-3 + 1e-5 * std::max(std::fabs(lo[a]), std::fabs(hi[a]));
-    fl[a] = std::nextafterf((float)(lo[a] - pad), -INFINITY);
-    fh[a] = std::nextafterf((float)(hi[a] + pad), INFINITY);
-  }
+  for (int a = 0; a < 3; a++) padBounds(lo[a], hi[a], planar, sizeof(R) == sizeof(float), fl[a], fh[a]);
   g.blo = make_float4(fl[0], fl[1], fl[2], 0.f); g.bhi = make_float4(fh[0], fh[1], fh[2], 0.f);
 }
 
@@ -94,7 +90,7 @@ Geom<R> rectGeom(int type, int owner, int flags, float eps, const RectD& r, floa
         pts[n_pts++] = r.A + r.e1 * ((d1 - c * d2) / den) + r.e2 * ((d2 - c * d1) / den);
       }
   }
-  setBounds(g, pts, n_pts, 0.0);
+  setBounds(g, pts, n_pts, 0.0, !(g.flags & GF_SPILL));   // a GF_SPILL region is as thin as the angle between its edges
   if (unbounded) { g.blo = make_float4(-1e30f, -1e30f, -1e30f, 0.f); g.bhi = make_float4(1e30f, 1e30f, 1e30f, 0.f); }
   return g;
 }
@@ -292,7 +288,7 @@ int flatten(const drt_prim* prims, int n_prims, const drt_light* lights, int n_l
         q.pA = cv<R>(V(p.center));
         Geom<R> g; memset(&g, 0, sizeof(g));
         g.type = G_SPHERE; g.owner = i; g.flags = 0; g.p0 = cv<R>(V(p.center)); g.f0 = (float)p.radius; g.vel = cv<R>(vel);
-        { const D3 pts[1] = {V(p.center)}; setBounds(g, pts, 1, (double)(float)p.radius); }
+        { const D3 pts[1] = {V(p.center)}; setBounds(g, pts, 1, (double)(float)p.radius, false); }
         hs.geoms.push_back(g);
         break; }
       case DRT_PRIM_CYLINDER: case DRT_PRIM_CHECKER_CYLINDER: {
@@ -307,7 +303,7 @@ int flatten(const drt_prim* prims, int n_prims, const drt_light* lights, int n_l
           g.flags |= GF_VERTEX_MOTION;
           g.len1 = (R)p.velocity2[0]; g.len2 = (R)p.velocity2[1]; g.pad_ = (R)p.velocity2[2];   // Geom::cylV2
         }
-        { const D3 pts[2] = {c1, c2}; setBounds(g, pts, 2, (double)(float)p.radius); }
+        { const D3 pts[2] = {c1, c2}; setBounds(g, pts, 2, (double)(float)p.radius, false); }
         hs.geoms.push_back(g);
         break; }
       case DRT_PRIM_TRIANGLE: {
@@ -318,7 +314,7 @@ int flatten(const drt_prim* prims, int n_prims, const drt_light* lights, int n_l
         Geom<R> g; memset(&g, 0, sizeof(g));
         g.type = G_TRI; g.owner = i; g.flags = (p.flags & DRT_FLAG_MESH) ? GF_MESH : 0;
         g.p0 = cv<R>(A); g.p1 = cv<R>(B - A); g.p2 = cv<R>(C - A); g.p3 = cv<R>(V(p.mesh_normal)); g.vel = cv<R>(vel);
-        { const D3 pts[3] = {A, B, C}; setBounds(g, pts, 3, 0.0); }
+        { const D3 pts[3] = {A, B, C}; setBounds(g, pts, 3, 0.0, true); }
         hs.geoms.push_back(g);
         break; }
       case DRT_PRIM_RECTANGLE: case DRT_PRIM_CHECKERBOARD: case DRT_PRIM_CHECKERBOARD_HOLE: {

@@ -533,8 +533,8 @@ __device__ inline bool geomIntersect(const Params<R>& P, const Geom<R>& g, int g
 
 // Conservative single-precision slab test against the geom's padded bounds: a cheap
 // filter in front of the exact (double) class test.  Never rejects a true hit: the
-// boxes are padded by 1e-3 + 1e-5*|coordinate| on the host and the comparison keeps a
-// relative margin, so only the cost -- not the candidate set -- changes.
+// boxes are padded beyond the rounding of the class's exact test (padBounds, drt_box.cuh)
+// and the comparison keeps a relative margin, so only the cost -- not the hits -- changes.
 __device__ inline bool slabMayHit(const float4 blo, const float4 bhi, const float nox, const float noy, const float noz,
                                   const float ix, const float iy, const float iz, const float t_limit, const float err) {
   // nox = -ox*ix etc. are hoisted per ray: each slab bound is one FFMA.  `err` bounds the

@@ -29,7 +29,8 @@ __device__ __forceinline__ uint64_t expandBits21(uint64_t v) {   // 21 bits -> e
   return v;
 }
 
-// per triangle: fp32 bounds (padded like the analytic geoms) + Morton code of the centroid.
+// per triangle: fp32 bounds + Morton code of the centroid.  The pad is the curved rule of padBounds (drt_box.cuh),
+// 1e-3 + 1e-5 |coordinate|, in float: padBounds says why mesh triangles do not take the planar pad.
 // The code cells are CUBES (`sinv` is one scale for all three axes: 1 / the largest extent) of 2^-21 of that extent.
 // With a scale per axis a flat mesh -- the terrain of config 5 is 12 x 2 x 12 -- spends every third level of the tree on a
 // split by height, whose two halves overlap almost everywhere in x and z (measured on that terrain: 32 % more node visits
