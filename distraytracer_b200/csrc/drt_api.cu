@@ -853,8 +853,9 @@ int planRender(drt_scene* s, const drt_settings* st, const drt_tile* tile, int& 
                            (long long)DRT_HITS_PER_PASS * (1 + (long long)st->max_depth * (fan - 1));
     if (need > (1ll << 22)) return fail(DRT_ERR_UNSUPPORTED, "brdf_samples * max_depth needs more than 4 M rays per CTA pool");
     // The pool is handed out in chunks of 32 slots.  On top of the chunks the pending rays fill: a chunk TRACE popped stays
-    // "in flight" until SHADE has consumed its hits (each holds at least one of the pass's hits), and every warp leaves at
-    // most one partly filled chunk behind per SHADE pass, which lives until the LIFO comes back to it.
+    // "in flight" until SHADE has consumed its hits (each holds at least one of the pass's hits), and a SHADE pass leaves at
+    // most one partly filled chunk behind, which lives until the LIFO comes back to it (`partial` allows DRT_WAVE_WARPS x 4
+    // of them per tree level).
     const long long live = (need + 31) / 32;
     const long long in_flight = std::min<long long>(live, DRT_CTA_HITS);
     const long long partial = (long long)DRT_WAVE_WARPS * 4 * (st->max_depth + 2);

@@ -19,6 +19,9 @@
 #include "drt_device.cuh"
 #include "drt_launch.h"
 #include <cstddef>
+#ifdef DRT_PASS_STATS
+#include <cstdio>
+#endif
 
 #ifndef DRT_FORCE_TREE
 #define DRT_FORCE_TREE 0   // diagnostic: 1 walks the replayed reference tree for every ray
@@ -1740,11 +1743,11 @@ __host__ __device__ constexpr size_t waveScratchBytes(int pool_cap) {
 // The pool is managed in CHUNKS of 32 slots (one bite of a warp).  A LIFO stack of chunk ids says which chunks hold
 // pending rays, a free list which ones are empty.  TRACE pops a chunk and traces its rays; a ray that hit something STAYS
 // in its slot and only a 16-byte reference (HitRef) goes to the hit buffer, so a chunk with hits is "in flight" until SHADE
-// has consumed them (a chunk without hits is free at once).  SHADE writes the children into chunks taken from the free
-// list -- every warp fills its own open chunk and pushes it when it is full -- and when the phase ends the chunks in
-// flight return to the free list.  (Round 1 copied every ray that hit into an 80-byte hit record: 64 more bytes
-// written to DRAM per hit, ~45 GB per bench frame.)  Slots a warp leaves unfilled in its last chunk of a phase are marked
-// empty (depth 0, which TRACE skips like the reference's `depth == 0` return).
+// has consumed them (a chunk without hits is free at once).  SHADE numbers the pass's children through one CTA-wide
+// cursor and writes them, 32 to a chunk, into chunks taken in order from the top of the free list, so a pass leaves at
+// most one partly filled chunk; when the phase ends the chunks in flight return to the free list.  (Round 1 copied every
+// ray that hit into an 80-byte hit record: 64 more bytes written to DRAM per hit, ~45 GB per bench frame.)  The unfilled
+// slots of the pass's last chunk are marked empty (depth 0, which TRACE skips like the reference's `depth == 0` return).
 template <typename R, int F, bool COUNT>
 __global__ void __launch_bounds__(32 * DRT_WAVE_WARPS, DRT_WAVE_CTAS_PER_SM) render_wave(const __grid_constant__ Params<R> P) {
   // dynamic shared memory: see s_dyn
@@ -1752,9 +1755,9 @@ __global__ void __launch_bounds__(32 * DRT_WAVE_WARPS, DRT_WAVE_CTAS_PER_SM) ren
   unsigned int* s_flags = (unsigned int*)(s_dyn + (size_t)DRT_CTA_SLOTS * 24);
   unsigned short* s_order = (unsigned short*)(s_dyn + (size_t)DRT_CTA_SLOTS * 28);
   unsigned char* s_hkey = s_dyn + (size_t)DRT_CTA_SLOTS * 28 + (size_t)DRT_CTA_HITS * 2;
-  // s_nst: chunks on the stack; s_nfree: chunks on the free list; s_ninfl: chunks in flight; s_npush: chunks SHADE pushed so far;
+  // s_nst: chunks on the stack; s_nfree: chunks on the free list; s_ninfl: chunks in flight; s_kid: children SHADE placed so far;
   // s_count: rays generated by a blur re-trace pass
-  __shared__ int s_nst, s_nfree, s_ninfl, s_npush, s_count, s_nhits, s_grab, s_state, s_nvalid;
+  __shared__ int s_nst, s_nfree, s_ninfl, s_kid, s_count, s_nhits, s_grab, s_state, s_nvalid;
   __shared__ int s_hist[DRT_HIT_BUCKETS];                 // SHADE order: counting sort of the hit buffer by geom
   __shared__ long long s_idx0, s_unit_next, s_unit_end;
   // slab-filter table of the whole scene, staged once per persistent CTA (48 B per pair of geoms)
@@ -1787,6 +1790,13 @@ __global__ void __launch_bounds__(32 * DRT_WAVE_WARPS, DRT_WAVE_CTAS_PER_SM) ren
   unsigned long long(*acc)[3] = s_acc;
   unsigned int* sfl = s_flags;
   const long long n_units = (P.sample_count + P.unit_samples - 1) / P.unit_samples;
+#ifdef DRT_PASS_STATS
+  // scheduling statistics of a diagnostic build (tools/pass_stats.py sums the lines printed at exit):
+  // [0] batches [1] passes [2] slots traced [3] of them empty [4] SHADE bites [5] partly filled chunks pushed
+  // [6] rays traced in the current pass [8 + b] TRACE passes whose ray count has bit length b (b = 0: none; 15: >= 16384)
+  __shared__ unsigned long long s_ps[24];
+  for (int i = tid; i < 24; i += blockDim.x) s_ps[i] = 0ull;
+#endif
 
   Counts cnt;
   if (COUNT) { cnt.samples = 0; cnt.rays = 0; cnt.shadow_rays = 0; cnt.shade_evals = 0; cnt.noise_evals = 0; cnt.node_tests = 0;
@@ -1795,7 +1805,7 @@ __global__ void __launch_bounds__(32 * DRT_WAVE_WARPS, DRT_WAVE_CTAS_PER_SM) ren
   // every chunk starts on the free list, lowest id on top
   for (int i = tid; i < n_chunks; i += blockDim.x) __stcg(fre + i, (uint32_t)(n_chunks - 1 - i));
   // s_state: 0 = no batch, 1 = primary trees in flight, 2 = blur re-traces in flight, 3 = all batches done
-  if (tid == 0) { s_nst = 0; s_nfree = n_chunks; s_ninfl = 0; s_npush = 0; s_count = 0; s_nhits = 0; s_state = 0; s_nvalid = 0;
+  if (tid == 0) { s_nst = 0; s_nfree = n_chunks; s_ninfl = 0; s_kid = 0; s_count = 0; s_nhits = 0; s_state = 0; s_nvalid = 0;
                   s_idx0 = 0; s_unit_next = 0; s_unit_end = 0; }
   __syncthreads();
 
@@ -1889,6 +1899,9 @@ __global__ void __launch_bounds__(32 * DRT_WAVE_WARPS, DRT_WAVE_CTAS_PER_SM) ren
             s_nvalid = (int)min((long long)DRT_CTA_SLOTS, end - next);
             s_unit_next = next + s_nvalid;
             s_state = 1;
+#ifdef DRT_PASS_STATS
+            s_ps[0]++;
+#endif
           }
         }
         __syncthreads();
@@ -1935,6 +1948,11 @@ __global__ void __launch_bounds__(32 * DRT_WAVE_WARPS, DRT_WAVE_CTAS_PER_SM) ren
       {
         Task<R> T;
         poolLoad<Task<R>, true>(T, pool, cap, slot);
+#ifdef DRT_PASS_STATS
+        const int n_empty = __popc(__ballot_sync(FULL, T.depth == 0));
+        if (lane == 0) { atomicAdd(&s_ps[2], 32ull); atomicAdd(&s_ps[3], (unsigned long long)n_empty);
+                         atomicAdd(&s_ps[6], (unsigned long long)(32 - n_empty)); }
+#endif
         if (T.depth != 0 && !(((volatile unsigned int*)sfl)[T.slot] & SF_ABORT)) {   // empty slot / an aborted sample spawns no more work (Q15)
           int motion;
           hit = traceRay<R, F, COUNT>(P, gb, T, h, motion, cnt);
@@ -1963,6 +1981,9 @@ __global__ void __launch_bounds__(32 * DRT_WAVE_WARPS, DRT_WAVE_CTAS_PER_SM) ren
     const int nst_base = max(s_grab, 0);                                 // untouched chunks stay at the bottom of the stack
     __syncthreads();
     if (tid == 0) s_grab = nh;
+#ifdef DRT_PASS_STATS
+    if (tid == 0) { s_ps[1]++; s_ps[8 + min(64 - __clzll((long long)s_ps[6]), 15)]++; s_ps[6] = 0ull; }
+#endif
     // ---- counting sort of the waiting hits by geom: the 32 hits a warp shades together then share
     // the material / model / texture branches of shadeA, evalBRDF and shadeB, and their shadow rays
     // leave from the same surface
@@ -1995,12 +2016,15 @@ __global__ void __launch_bounds__(32 * DRT_WAVE_WARPS, DRT_WAVE_CTAS_PER_SM) ren
     __syncthreads();
 
     // ================= SHADE: waiting hits -> radiance terms + child rays ====================
-    int open_id = -1, open_fill = 0;                                     // the warp's partly filled chunk of children (warp-uniform)
+    const int f0 = s_nfree;                                              // the free list holds still while SHADE runs
     for (;;) {
       int end = 0;
       if (lane == 0) end = atomicSub(&s_grab, 32);
       end = __shfl_sync(FULL, end, 0);
       if (end <= 0) break;
+#ifdef DRT_PASS_STATS
+      if (lane == 0) atomicAdd(&s_ps[4], 1ull);
+#endif
       const int begin = max(end - 32, 0);
       const int take = end - begin;
       const bool active = lane < take;
@@ -2018,6 +2042,9 @@ __global__ void __launch_bounds__(32 * DRT_WAVE_WARPS, DRT_WAVE_CTAS_PER_SM) ren
         HitRec h; h.t = __uint_as_float(hr.x); h.geom = (int)hr.y; h.inside = (int)(hr.z & 1u); h.checker_sel = (int)(hr.z >> 1);
         slot = T.slot;
         shadeA<R, F, COUNT>(P, T, h, kids, nk, add, has_add, aborted, S, cnt);
+        // children of depth 0 return at once (traceRay, :489) without touching the sample's flags: they are not placed,
+        // so TRACE's chunks hold only rays it traces
+        if (T.depth == 1) nk = 0;
         if (!aborted && S.lights) { pin.isectP = S.isectP; pin.path = T.path; pin.val = S.mv.val; pin.dt = T.dt; pin.want = 1; }
       }
       // -- step B (lane = (hit, light) pair): light sample + shadow ray, DRT_PAIR_LIGHTS lights at a time; a pair lane
@@ -2061,57 +2088,59 @@ __global__ void __launch_bounds__(32 * DRT_WAVE_WARPS, DRT_WAVE_CTAS_PER_SM) ren
           if (orf) atomicOr(&sfl[slot], orf);
         }
       }
-      // the children go into the warp's open chunk and on into fresh chunks from the free list, child-index-major: the
-      // j-th children of the warp's 32 (geom-sorted) hits -- the same kind of ray leaving the same surface -- end up
-      // adjacent, so a later TRACE warp works on rays with similar candidates
+      // the bite's children take the next `total` numbers of the pass's child cursor, child-index-major: the j-th children
+      // of the warp's 32 (geom-sorted) hits -- the same kind of ray leaving the same surface -- end up adjacent, so a later
+      // TRACE warp works on rays with similar candidates.  Child v goes to lane v & 31 of chunk c = v >> 5, the c-th chunk
+      // from the top of the free list, which the bite that writes its lane 0 puts on the stack at nst_base + c.
       const int total = __reduce_add_sync(FULL, nk);
       if (total) {
-        const int have = open_id >= 0 ? 1 : 0;                            // open_fill is 0 without an open chunk
-        const int touched = (open_fill + total + 31) >> 5;                // chunks written to: the open one (if any), then new ones
-        const int fresh = touched - have;
-        int f = 0;
-        if (lane == 0 && fresh) f = atomicSub(&s_nfree, fresh);
-        f = __shfl_sync(FULL, f, 0);
-        if (fresh && f < fresh) {                                         // cannot happen within the validated bounds
-          if (nk) atomicOr(&sfl[kids[0].slot], SF_ABORT);
-          if (lane == 0) { *P.overflow = 1; atomicAdd(&s_nfree, fresh); }
-        } else {
-          int myid = -1;                                                  // lane k: id of the k-th chunk written to
-          if (lane < touched) myid = (have && lane == 0) ? open_id : (int)__ldcg(fre + f - 1 - (lane - have));
-          int base = open_fill;
+        int base = 0;
+        if (lane == 0) base = atomicAdd(&s_kid, total);
+        base = __shfl_sync(FULL, base, 0);
+        const int c0 = base >> 5, room = 32 * f0;                         // the bite's first chunk; child slots the free list holds
+        if (lane == 0 && base + total > room) *P.overflow = 1;            // cannot happen within the validated bounds
+        int myid = 0;                                                     // lane k: id of chunk c0 + k
+        if (lane <= ((base + total - 1) >> 5) - c0 && c0 + lane < f0) {
+          myid = (int)__ldcg(fre + f0 - 1 - (c0 + lane));
+          if (((c0 + lane) << 5) >= base) __stcg(stk + nst_base + c0 + lane, (uint32_t)myid);
+        }
 #pragma unroll 1
-          for (int j = 0; j < DRT_MAX_CHILDREN; j++) {                    // a rolled loop: the bench workload has at most 3 children per hit
-            const unsigned int kbj = __ballot_sync(FULL, nk > j);
-            if (!kbj) break;
-            const int g = base + __popc(kbj & ((1u << lane) - 1u));
-            const int cid = __shfl_sync(FULL, myid, (nk > j) ? (g >> 5) : 0);
-            if (nk > j) poolStore(pool, cap, cid * 32 + (g & 31), kids[j]);
-            base += __popc(kbj);
+        for (int j = 0; j < DRT_MAX_CHILDREN; j++) {                      // a rolled loop: the bench workload has at most 3 children per hit
+          const unsigned int kbj = __ballot_sync(FULL, nk > j);
+          if (!kbj) break;
+          const int g = base + __popc(kbj & ((1u << lane) - 1u));
+          const int cid = __shfl_sync(FULL, myid, (nk > j) ? (g >> 5) - c0 : 0);
+          if (nk > j) {
+            if (g < room) poolStore(pool, cap, cid * 32 + (g & 31), kids[j]);
+            else atomicOr(&sfl[kids[j].slot], SF_ABORT);                  // overflow: the sample is aborted, the frame rejected
           }
-          const int full = base >> 5;                                     // chunks completed by this bite
-          int pp = 0;
-          if (lane == 0 && full) pp = atomicAdd(&s_npush, full);
-          pp = __shfl_sync(FULL, pp, 0);
-          if (lane < full) __stcg(stk + nst_base + pp + lane, (uint32_t)myid);
-          open_fill = base & 31;
-          open_id = __shfl_sync(FULL, myid, min(full, 31));
-          if (!open_fill) open_id = -1;
+          base += __popc(kbj);
         }
       }
     }
-    if (open_id >= 0) {                                                  // the warp's last chunk of this pass: mark the unused slots, push it
-      if (lane >= open_fill) poolStoreEmpty<Task<R>>(pool, cap, open_id * 32 + lane);
-      if (lane == 0) __stcg(stk + nst_base + atomicAdd(&s_npush, 1), (uint32_t)open_id);
-    }
     __syncthreads();
-    {                                                                    // the chunks in flight are consumed: back to the free list
-      const int ninfl = s_ninfl, f = s_nfree;
-      for (int i = tid; i < ninfl; i += blockDim.x) __stcg(fre + f + i, __ldcg(infl + i));
+    {  // the children's chunks have left the free list (the unused slots of the last one are marked empty), and the chunks
+       // in flight are consumed: back to the free list
+      const int nkid = s_kid, nch = min((nkid + 31) >> 5, f0), ninfl = s_ninfl;
+      if (nkid < nch * 32) {
+        const int last = (int)__ldcg(stk + nst_base + nch - 1);
+        for (int q = nkid + tid; q < nch * 32; q += blockDim.x) poolStoreEmpty<Task<R>>(pool, cap, last * 32 + (q & 31));
+      }
+      for (int i = tid; i < ninfl; i += blockDim.x) __stcg(fre + f0 - nch + i, __ldcg(infl + i));
       __syncthreads();
-      if (tid == 0) { s_nfree = f + ninfl; s_ninfl = 0; s_nst = nst_base + s_npush; s_npush = 0; s_nhits = 0; }
+      if (tid == 0) { s_nfree = f0 - nch + ninfl; s_ninfl = 0; s_nst = nst_base + nch; s_kid = 0; s_nhits = 0; }
+#ifdef DRT_PASS_STATS
+      if (tid == 0 && nkid < nch * 32) s_ps[5]++;
+#endif
     }
     __syncthreads();
   }
+#ifdef DRT_PASS_STATS
+  if (tid == 0)   // one printf per CTA, so that the lines of different CTAs do not interleave
+    printf("PASS_STATS %d %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu\n",
+           blockIdx.x, s_ps[0], s_ps[1], s_ps[2], s_ps[3], s_ps[4], s_ps[5], s_ps[8], s_ps[9], s_ps[10], s_ps[11], s_ps[12],
+           s_ps[13], s_ps[14], s_ps[15], s_ps[16], s_ps[17], s_ps[18], s_ps[19], s_ps[20], s_ps[21], s_ps[22], s_ps[23]);
+#endif
 
   if (COUNT) {
     atomicAdd(&P.counts->samples, cnt.samples); atomicAdd(&P.counts->rays, cnt.rays);
