@@ -312,6 +312,175 @@ def random_glass_scene(seed):
     return "random_glass", Scene(extra + prims, lights, scene.textures), s
 
 
+# ---- sized scenes: the same picture with more or fewer scene records -------------------------------------------------
+# render_wave's launcher picks its instantiation by scene size (csrc/drt_launch.h): more than SMEM_GEOMS geoms sets FT_BIG
+# (the geom tree, or the global slab table when a slab-box prism is present), and records of more than SMEM_RECS bytes are
+# read from global memory instead of the CTA's shared copy (no FT_RECS).  Bytes of one Geom<R>, PrimD<R>, LightD<R> record
+# per precision (drt_settings.precision: 0 double, 1 float); a mesh's material table adds one PrimD per entry.
+SMEM_GEOMS, SMEM_RECS = 256, 32 * 1024
+RECORD_BYTES = {0: (224, 1280, 160), 1: (160, 784, 96)}
+SIZED_KINDS = ("scene", "textured", "motion", "glass", "refblur", "prism", "mesh", "moving_mesh")
+ENCLOSURE_CENTER, ENCLOSURE_RADIUS = (24.0, 1.0, 0.0), 3.0
+
+
+def geom_count(prims):
+    """Geoms flatten (csrc/drt_api.cu) makes of `prims`: one per primitive, two for a checkerboard with a hole (board and
+    hole), six for a RectPrismV2 (its faces)."""
+    from distraytracer_b200 import abi
+    return sum(2 if p.type == abi.PRIM_CHECKERBOARD_HOLE else 6 if p.type == abi.PRIM_RECTPRISMV2 else 1 for p in prims)
+
+
+def mesh_materials(scene):
+    """Entries of the mesh's material table (0 without a mesh; 1 when every triangle takes drt_mesh.material)."""
+    if scene.mesh is None:
+        return 0
+    return len(scene.mesh.get("materials") or []) or 1
+
+
+def record_bytes(scene, precision):
+    """Bytes of the geom, primitive and light records render_wave stages in shared memory when they fit."""
+    g, p, l = RECORD_BYTES[precision]
+    return g * geom_count(scene.prims) + p * (len(scene.prims) + mesh_materials(scene)) + l * len(scene.lights)
+
+
+def _filler(rng, geoms):
+    """One small opaque shape of `geoms` geoms (1: sphere, cylinder, rectangle or triangle; 2: checkerboard with a hole;
+    6: RectPrismV2) somewhere inside the enclosing sphere."""
+    from distraytracer_b200 import abi, scenes
+    c = np.asarray(ENCLOSURE_CENTER) + rng.uniform(-0.35, 0.35, 3) * ENCLOSURE_RADIUS
+    col = tuple(rng.uniform(0.2, 1.0, 3))
+    s = float(rng.uniform(0.05, 0.2))
+    if geoms == 1:
+        kind = int(rng.integers(4))
+        if kind == 0:
+            return scenes.sphere(c, s, col)
+        if kind == 1:
+            return scenes.cylinder(c, c + rng.normal(0, s, 3), 0.3 * s, col)
+        if kind == 2:
+            return scenes.triangle(c, c + rng.normal(0, s, 3), c + rng.normal(0, s, 3), col)
+        return scenes.rectangle(c, c + (s, 0, 0), c + (s, s, 0), c + (0, s, 0), col, name=abi.NAME_OTHER)
+    if geoms == 2:
+        p = scenes.checkerboard(c, c + (0, 0, s), c + (s, 0, s), c + (s, 0, 0), col, (0.1, 0.1, 0.1), 0.05)
+        p.type = abi.PRIM_CHECKERBOARD_HOLE
+        q = 0.25 * s
+        for dst, v in zip(p.hole, (c + (q, 0, q), c + (q, 0, 3 * q), c + (3 * q, 0, 3 * q), c + (3 * q, 0, q))):
+            dst[:] = list(v)
+        return p
+    assert geoms == 6
+    p = scenes.new_prim(); p.type = abi.PRIM_RECTPRISMV2
+    A, B, C, D = c, c + (0, 0, s), c + (0, s, s), c + (0, s, 0)
+    for dst, v in zip((p.A, p.B, p.C, p.D, p.E, p.F, p.G, p.H), (A, B, C, D, A + (s, 0, 0), B + (s, 0, 0), C + (s, 0, 0), D + (s, 0, 0))):
+        dst[:] = list(v)
+    p.color[:] = list(col); p.center[:] = list(c + 0.5 * s)
+    return p
+
+
+def _base(kind, seed):
+    """-> (name, scene for the CUDA path, the same with the mesh as Triangle primitives or None, settings)."""
+    from distraytracer_b200 import abi, scenes
+    from distraytracer_b200.scene import Scene
+    flat = None
+    if kind in ("scene", "textured"):
+        name, scene, s = random_scene(seed)
+        if kind == "textured":              # a textured floor under the shapes (FT_TEX)
+            floor = scenes.rectangle((-8, -3.5, 8), (8, -3.5, 8), (8, -3.5, -8), (-8, -3.5, -8), (0.7, 0.7, 0.7),
+                                     tex_frame=0, name=abi.NAME_OTHER)
+            floor.flags |= abi.FLAG_TEXTURE
+            scene = Scene(scene.prims + [floor], scene.lights, scene.textures)
+    elif kind == "motion":
+        name, scene, s = random_motion_scene(seed)
+    elif kind == "glass":
+        name, scene, s = random_glass_scene(seed)
+    elif kind == "refblur":
+        name, scene, s = random_refblur_scene(seed)
+    elif kind == "prism":
+        name, scene, s = random_prism_scene(seed)
+    elif kind == "mesh":
+        name, scene, flat, s = random_mesh_scene(seed)
+    else:
+        assert kind == "moving_mesh", kind
+        name, scene, flat, s = random_moving_mesh_scene(seed)
+    return name, scene, flat, s
+
+
+def sized_scene(kind, seed, precision=0, geoms=None, recs=None, recs_at_most=False, extra_materials=0, frame_range=None,
+                twins=False):
+    """A base scene drawn like random_scene / random_mesh_scene / ... (`kind`, one of SIZED_KINDS) plus an opaque enclosing
+    sphere on the +x side, far from the camera and the shapes, and "filler": small shapes inside that sphere.  No camera,
+    reflection, refraction or shadow ray reaches the filler (each one crosses the sphere first), so the filler changes the
+    scene's tables but not its picture.  The filler goes after every other primitive (area lights keep their prim_index);
+    in the reference's candidate order it comes first, so the base scene's geoms keep the end of the slab table.
+
+    geoms: add 1-geom filler up to that many geoms in all.  recs: add filler (spheres, checkerboards with a hole, RectPrismV2)
+    up to exactly that many record bytes in `precision` (recs_at_most: the most the filler can make without exceeding
+    `recs`; the byte counts it can add are combinations of three record sizes).  extra_materials: entries appended to the
+    mesh's material table, which no triangle uses.  frame_range: override (velocity blur: 1 keeps the swept boxes, more re-traces unfiltered).
+    twins: every rectangle and triangle of the base gets a coplanar copy of another colour, appended (exact ties of t: the
+    first in the reference's candidate order must win).
+    -> (name, scene, flat, settings); `flat` is the scene the oracle takes (mesh triangles as Triangle primitives)."""
+    from distraytracer_b200 import abi, scenes
+    from distraytracer_b200.scene import Scene
+    name, scene, flat, s = _base(kind, seed)
+    rng = np.random.default_rng(123000 + seed)
+    s.xRes, s.yRes = min(s.xRes, 64), min(s.yRes, 48)
+    s.antialias_samples = min(s.antialias_samples, 4)
+    if frame_range is not None:
+        s.frame_range = frame_range
+    prims = [abi.copy_struct(p) for p in scene.prims]
+    if twins:
+        for p in scene.prims:
+            if p.type in (abi.PRIM_RECTANGLE, abi.PRIM_TRIANGLE) and not (p.flags & abi.FLAG_LIGHT):
+                q = abi.copy_struct(p); q.color[:] = [1.0 - x for x in p.color]; prims.append(q)
+    prims.append(scenes.sphere(ENCLOSURE_CENTER, ENCLOSURE_RADIUS, (0.55, 0.5, 0.45)))
+    mesh = dict(scene.mesh) if scene.mesh is not None else None
+    if extra_materials:
+        assert mesh is not None, "extra_materials needs a mesh"
+        mats = list(mesh.get("materials") or [mesh["material"]])
+        if not mesh.get("materials"):
+            mesh["material_ids"] = np.zeros(len(mesh["indices"]), dtype=np.int32)
+        mesh["materials"] = mats + [abi.copy_struct(mats[0]) for _ in range(extra_materials)]
+    def sized(extra):
+        return Scene(prims + extra, scene.lights, scene.textures, mesh=mesh)
+    extra = []
+    if geoms is not None:
+        n = geoms - geom_count(prims)
+        assert n >= 0, (kind, seed, "base scene has more geoms than", geoms)
+        extra = [_filler(rng, 1) for _ in range(n)]
+    if recs is not None:
+        G, P, _ = RECORD_BYTES[precision]
+        base = record_bytes(sized([]), precision)
+        plan = None
+        for target in range(recs, base - 1, -16) if recs_at_most else (recs,):
+            need = target - base
+            plan = next(((n1, n2, n6) for n6 in range(12) for n2 in range(5)
+                         for n1 in [(need - n6 * (6 * G + P) - n2 * (2 * G + P)) // (G + P)]
+                         if n1 >= 0 and n1 * (G + P) + n2 * (2 * G + P) + n6 * (6 * G + P) == need), None)
+            if plan is not None:
+                break
+        assert plan is not None, (kind, seed, "no filler makes", recs, "record bytes from", base)
+        extra += [_filler(rng, g) for g, k in zip((1, 2, 6), plan) for _ in range(k)]
+    out = sized(extra)
+    if recs is not None:
+        assert record_bytes(out, precision) == target
+    if flat is not None:
+        flat = Scene(prims + extra + scenes.mesh_to_prims(mesh), scene.lights, scene.textures)
+    return f"{name}+{kind}", out, flat if flat is not None else out, s
+
+
+def one_more_record(scene, seed=0):
+    """The scene of sized_scene with one more record and the same picture: one more unused entry in the mesh's material
+    table, or, without a mesh, one more 1-geom filler shape.  -> (scene, flat)."""
+    from distraytracer_b200 import abi, scenes
+    from distraytracer_b200.scene import Scene
+    if scene.mesh is not None:
+        mesh = dict(scene.mesh)
+        mesh["materials"] = list(mesh["materials"]) + [abi.copy_struct(mesh["materials"][0])]
+        more = Scene(scene.prims, scene.lights, scene.textures, mesh=mesh)
+        return more, Scene(scene.prims + scenes.mesh_to_prims(mesh), scene.lights, scene.textures)
+    more = Scene(scene.prims + [_filler(np.random.default_rng(124000 + seed), 1)], scene.lights, scene.textures)
+    return more, more
+
+
 def random_refblur_scene(seed):
     """random_scene in the REFERENCE's blur mode after frame_prism: shapes named "rectangle" move in y during the blur
     re-traces of samples that hit a primitive flagged `motion` (render_final_project.cpp:1095-1210), leaf boxes are widened

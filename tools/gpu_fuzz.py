@@ -1,7 +1,7 @@
 """GPU vs oracle on mutated fixture scenes, any number of seeds (tests/test_gpu_parity.py runs the first 14).
   python tools/gpu_fuzz.py [n_cases] [cam]
 `scenes`: random scenes instead of mutated fixtures (random_scene); `meshes`: random triangle meshes (random_mesh_scene); `motion`: random scenes in velocity-blur mode (random_motion_scene); `big`: more than 256 shapes (random_big_scene);
-`sky`: mutated fixtures in front of the value-noise clouds (sky_case); `meshmotion`: a moving mesh in velocity-blur mode; `prisms`: random slab-box prisms with holes (random_prism_scene); `glass`: random scenes with glass blocks; `refblur`: random scenes in the reference's own blur mode.  `cam`: the camera is moved as well (eye / lookingAt jittered, focal length and aperture redrawn), so rays reach the scenes
+`sky`: mutated fixtures in front of the value-noise clouds (sky_case); `meshmotion`: a moving mesh in velocity-blur mode; `prisms`: random slab-box prisms with holes (random_prism_scene); `glass`: random scenes with glass blocks; `refblur`: random scenes in the reference's own blur mode; `sizes`: fuzz_cases.sized_scene -- a random kind pushed to 255 / 256 / 257 geoms, 257..400 geoms or records just under the shared-memory bound.  `cam`: the camera is moved as well (eye / lookingAt jittered, focal length and aperture redrawn), so rays reach the scenes
 from directions the reference's builders never look from -- grazing walls, looking along an axis, from inside a prism.
 """
 import os
@@ -9,7 +9,7 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
-from fuzz_cases import mutated_case, random_scene, random_mesh_scene, random_motion_scene, random_big_scene, sky_case, random_moving_mesh_scene, random_prism_scene, random_glass_scene, random_refblur_scene  # noqa: E402
+from fuzz_cases import mutated_case, random_scene, random_mesh_scene, random_motion_scene, random_big_scene, sky_case, random_moving_mesh_scene, random_prism_scene, random_glass_scene, random_refblur_scene, sized_scene, SIZED_KINDS, SMEM_RECS  # noqa: E402
 from distraytracer_b200 import runtime  # noqa: E402
 from oracle.harness import Oracle, ORACLE_KEYED, compare  # noqa: E402
 
@@ -28,6 +28,17 @@ for seed in range(n_cases):
     elif len(sys.argv) > 2 and sys.argv[2] == "prisms": case, sc, s = random_prism_scene(seed)
     elif len(sys.argv) > 2 and sys.argv[2] == "glass": case, sc, s = random_glass_scene(seed)
     elif len(sys.argv) > 2 and sys.argv[2] == "refblur": case, sc, s = random_refblur_scene(seed)
+    elif len(sys.argv) > 2 and sys.argv[2] == "sizes":
+        import numpy as np
+        rng = np.random.default_rng(78000 + seed)
+        kind = SIZED_KINDS[int(rng.integers(len(SIZED_KINDS)))]
+        size = int(rng.integers(4))
+        kw = dict(geoms=int(rng.choice([255, 256, 257]))) if size == 0 else dict(geoms=int(rng.integers(257, 401))) if size == 1 else \
+            dict(recs=SMEM_RECS, recs_at_most=True, precision=int(os.environ.get("DRT_FUZZ_PRECISION", "0"))) if size == 2 else {}
+        try:
+            case, sc, flat, s = sized_scene(kind, seed, **kw)
+        except AssertionError:                          # base already past the requested size
+            case, sc, flat, s = sized_scene(kind, seed)
     else: case, sc, s = random_scene(seed) if random_scenes else mutated_case(seed)
     if move_camera:
         import numpy as np
